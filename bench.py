@@ -1,7 +1,8 @@
 #!/usr/bin/env python3
 """bench.py -- SMEM reads/s on B200 (BASELINE.json metric) for the B200-native engine.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c4|c3|c5] [--scaling strong|weak] [--impl reference] ...
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c4|c3|c5] [--scaling strong|weak] [--impl reference]
+                    [--dump-outputs DIR] ...
 
 Workload = BASELINE.json configs[3] (`--config c4`, the configuration the metric is quoted on): synthetic 1 Gbp random ACGT
 reference (numpy PCG64(1000)), 50 M reads of 151 bp (exact substrings with i.i.d. 1 % substitutions, SURVEY 8d), all three
@@ -35,6 +36,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from, which may be read-only
 
 READ_LEN = 151
 SUB_RATE = 0.01
@@ -195,6 +197,11 @@ CONFIGS = {"c4": dict(ref_bases=1_000_000_000, reads=50_000_000, seed=1000, expe
            "c5": dict(ref_bases=3_000_000_000, reads=100_000_000, seed=3000, experts=(4096, 4194304), name="BASELINE.json configs[4]")}
 HOST_READS = 600_000      # the first reads of every batch come from numpy so the CPU arms can regenerate exactly them
 PARITY_READS = 20_000     # reads per method compared with the oracle at N = 1 (2,048 at N > 1)
+# --dump-outputs: reads sampled with a fixed seed.  A read has at most READ_LEN records (their ends strictly increase), so
+# 10,000 reads x 151 records x 40 bytes (5 float64 fields) keeps the dump under 64 MB whatever the workload.
+DUMP_READS = 10_000
+DUMP_SEED = 20261020
+DUMP_MAX_BYTES = 64_000_000
 
 
 def parse_args():
@@ -214,7 +221,13 @@ def parse_args():
     ap.add_argument("--seed-k", type=int, default=-1, help="K of the sweep kernel's seed table (-1 = auto, 0 = none)")
     ap.add_argument("--sub-rate", type=float, default=SUB_RATE, help="substitution rate of the synthetic reads (SURVEY 8d extremes: 0)")
     ap.add_argument("--random-reads", action="store_true", help="uniform random reads instead of reference substrings (SURVEY 8d extreme)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed BWA-SMEM step returned in its last step (a fixed sample of reads) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native path")
     cfg = dict(CONFIGS[args.config])
     if args.ref_bases:
         cfg["ref_bases"] = args.ref_bases
@@ -285,6 +298,34 @@ def algorithmic_bytes(recs_i32, n_rec, n_reads, K=0, probe_bytes=0):
     return total, steps, n_long
 
 
+def dump_outputs(out_dir, engine, n_reads, n_mems, n_rec):
+    """What Engine.run hands its caller for the batch the engine just ran (records, CSR offsets, per-read status, counts),
+    for DUMP_READS reads drawn with DUMP_SEED, as float64 arrays in out_dir:
+      read_ids (S,)      the sampled reads, ascending
+      status   (S,)      READ_OK / READ_REF_RAISES / READ_TOO_SHORT of each sampled read
+      offsets  (S + 1,)  CSR offsets of the sampled reads' rows in `records`
+      records  (R, 5)    read_id, qstart, qend, sa_lo, sa_hi
+      totals   (2,)      maximal matches and records of the whole batch"""
+    import torch
+    from genie_smem_b200.engine import RECORD_DTYPE
+    dev = engine.device
+    ids = np.sort(np.random.default_rng(DUMP_SEED).choice(n_reads, min(n_reads, DUMP_READS), replace=False))
+    ids_t = torch.from_numpy(ids).to(dev)
+    lo = engine.rec_off[ids_t].cpu().numpy()
+    hi = engine.rec_off[ids_t + 1].cpu().numpy()
+    rows = torch.from_numpy(np.concatenate([np.arange(a, b) for a, b in zip(lo, hi)] + [np.empty(0, np.int64)])).to(dev)
+    recs = engine.records[: n_rec * 16].view(torch.int32).view(-1, 4)[rows].cpu().numpy().view(RECORD_DTYPE).reshape(-1)
+    arrays = {"read_ids": ids, "status": engine.read_status[ids_t].cpu().numpy(), "offsets": np.concatenate([[0], np.cumsum(hi - lo)]),
+              "records": np.stack([recs[f] for f in RECORD_DTYPE.names], axis=1), "totals": np.asarray([n_mems, n_rec])}
+    arrays = {k: np.asarray(v, np.float64) for k, v in arrays.items()}
+    nbytes = sum(a.nbytes for a in arrays.values())
+    assert nbytes <= DUMP_MAX_BYTES, f"output dump of {nbytes} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    log(f"outputs of the last timed step: {len(ids)} reads, {len(recs)} records, {nbytes / 1e6:.1f} MB in {out_dir}")
+
+
 def main():
     args = parse_args()
     _claim_stdout()
@@ -304,6 +345,8 @@ def main():
     from genie_smem_b200 import sharding
 
     assert torch.cuda.is_available(), "bench.py needs a CUDA device (no CPU fallback)"
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs runs on one GPU")
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     if world > 1:
@@ -423,6 +466,8 @@ def main():
     t_region1 = time.time()
     clocks = sampler.stop(t_region0, t_region1)
     n_mems, n_rec = engine.check_overflow()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, engine, n_reads, n_mems, n_rec)
     gathered = None
     if gat is not None:
         parts, totals = gat.finish()
@@ -799,7 +844,7 @@ def python_port_baseline(budget_s=1.5):
     process that never touched CUDA."""
     try:
         r = subprocess.run([sys.executable, "-m", "oracle.py_baseline", "--seconds", str(budget_s)], cwd=ROOT, capture_output=True,
-                           text=True, timeout=120)
+                           text=True, timeout=120, env=dict(os.environ, PYTHONDONTWRITEBYTECODE="1"))
         if r.returncode != 0:
             return {"unavailable": (r.stderr or "oracle.py_baseline failed").strip().splitlines()[-1][:200]}
         return json.loads(r.stdout.strip().splitlines()[-1])

@@ -123,20 +123,17 @@ def test_rmi_big_k15_fit_matches_reference_trained_parameters():
 
 def test_rmi_lut_save_in_reference_format_is_loadable_as_the_reference_class(workdir):
     """reference_format=True pickles an RMI.RMI whose .models hold sklearn LinearRegression objects (what RMI_LUT.load of the
-    reference unpickles, RMI_LUT.py:192-198); with the real reference on this machine its own predict() is run on it."""
+    reference unpickles, RMI_LUT.py:192-198).  Routing k-mers through those models as the reference's RMI.predict does
+    (RMI.py:52-69) gives, bit for bit, the predictions the reference made with the same model
+    (tests/golden/rmi_lookups_medium_data_k6.json.gz)."""
     import genie_smem_b200 as gs
     tmp, g = workdir
     m = gs.ExactMatch.from_text(g["text"], suffix_array=g["suffix_array"], name="medium_data.fa")
     p = gu.load_rmi("medium_data_k6")
     r = gs.RMI_LUT(p["experts"], 6, "medium_data.fa", matcher=m)
     r.rmi = gs.RMI.from_params(p["level_sizes"], p["coef"], p["intercept"])
-    ref_dir = "/root/reference/SMEM"
     had = sys.modules.pop("RMI", None)
     try:
-        if os.path.exists(os.path.join(ref_dir, "RMI.py")):
-            sys.path.insert(0, ref_dir)
-            import RMI as ref_rmi_module                    # the reference's own class  # noqa: F401
-            sys.path.remove(ref_dir)
         r.save("ref_style.pkl", reference_format=True)
         with open("ref_style.pkl", "rb") as f:
             structure, K, data_file, obj = pickle.load(f)   # plain pickle.load, as the reference does
@@ -144,9 +141,18 @@ def test_rmi_lut_save_in_reference_format_is_loadable_as_the_reference_class(wor
         assert type(obj).__module__ == "RMI" and type(obj).__name__ == "RMI"
         assert [len(l) for l in obj.models] == p["level_sizes"]
         assert float(obj.models[1][3].coef_[0]) == float(p["coef"][4]) and float(obj.models[1][3].intercept_) == float(p["intercept"][4])
-        if hasattr(obj, "predict"):                         # the reference's RMI.predict (RMI.py:52-69) on our pickle
-            keys = np.arange(0, 4 ** 6, 37, dtype=np.int64).reshape(-1, 1)
-            assert np.array_equal(np.asarray(obj.predict(keys)).reshape(-1), r.rmi.predict(keys.reshape(-1)))
+        rows = [row for row in gu.load_json("rmi_lookups_medium_data_k6.json.gz") if row[1] is not None]
+        assert len(rows) > 2000
+        scales = [len(l) for l in obj.models[1:]] + [1]
+        for q, ref_pred, _, _ in rows:
+            x = np.asarray([[gs.LUT.convert_seq_to_num(q)]], np.float64)
+            k = 0
+            for level, scale in zip(obj.models, scales):
+                y = float(level[k].predict(x)[0])
+                k = min(scale - 1, max(0, int(y)))
+            assert y == ref_pred, q
+        keys = np.asarray([gs.LUT.convert_seq_to_num(row[0]) for row in rows], np.int64)
+        assert np.array_equal(r.rmi.predict(keys), np.asarray([row[1] for row in rows]))
         back = gs.RMI_LUT.load("ref_style.pkl", matcher=m)   # and this package reads it back
         assert np.array_equal(back.rmi.coef, p["coef"]) and np.array_equal(back.rmi.intercept, p["intercept"])
     finally:
