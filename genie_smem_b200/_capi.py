@@ -51,6 +51,16 @@ class WorkspaceInfo(C.Structure):
     _fields_ = [("quad_scratch_bytes", C.c_uint64), ("scan_tmp_bytes", C.c_uint64), ("grid_blocks", C.c_uint32), ("block_threads", C.c_uint32)]
 
 
+class DevContigs(C.Structure):
+    _fields_ = [("n", C.c_uint64), ("start", C.c_void_p)]
+
+
+class Hit(C.Structure):
+    _fields_ = [("record", C.c_uint32), ("contig", C.c_uint32), ("offset", C.c_uint32), ("flags", C.c_uint32)]
+
+
+HIT_SPANS, HIT_SAMPLED = 1, 2
+
 EXPORTS = {
     # name: (restype, argtypes)
     "gsm_index_build": (C.c_int, [C.c_char_p, C.c_uint64, C.c_uint32, C.POINTER(C.c_void_p)]),
@@ -114,6 +124,10 @@ EXPORTS = {
     "gsm_device_l2_fetch_granularity": (C.c_int, [C.c_int32, C.POINTER(C.c_uint32)]),
     "gsm_last_error": (C.c_char_p, []),
     "gsm_version": (C.c_int, []),
+    "gsm_hits_workspace_info": (C.c_int, [C.c_uint64, C.POINTER(C.c_uint64)]),
+    "gsm_hits_count": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
+    "gsm_hits_locate": (C.c_int, [C.POINTER(DevIndex), C.c_void_p, C.c_uint32, C.POINTER(DevContigs), C.c_void_p, C.c_void_p, C.c_uint64,
+                                  C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
 }
 
 

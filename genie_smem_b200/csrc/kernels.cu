@@ -1266,6 +1266,24 @@ int launch_seeded(const SelectArgs& se, int cap, cudaStream_t stream) {
 
 }  // namespace
 
+uint64_t gsm::scan_tmp_bytes(uint64_t n) { return ((n + SCAN_TILE - 1) / SCAN_TILE + 2) * 8ull; }
+
+int gsm::scan_counts(const uint32_t* cnt, uint64_t n, uint64_t* off, void* tmp, uint64_t tmp_bytes, void* stream) {
+    cudaStream_t s = (cudaStream_t)stream;
+    if (n == 0) {
+        GSM_CUDA(cudaMemsetAsync(off, 0, sizeof(uint64_t), s));
+        return GSM_OK;
+    }
+    if (tmp_bytes < scan_tmp_bytes(n)) return fail(GSM_E_CAPACITY, "scan_tmp too small");
+    const uint64_t n_tiles = (n + SCAN_TILE - 1) / SCAN_TILE;
+    unsigned long long* tiles = (unsigned long long*)tmp;
+    k_scan_tiles<<<(unsigned)n_tiles, SCAN_THREADS, 0, s>>>(cnt, n, (unsigned long long*)off, tiles);
+    k_scan_top<<<1, SCAN_THREADS, 0, s>>>(tiles, n_tiles, tiles + n_tiles);
+    k_scan_add<<<(unsigned)n_tiles, SCAN_THREADS, 0, s>>>((unsigned long long*)off, n, tiles, tiles + n_tiles);
+    GSM_CUDA(cudaGetLastError());
+    return GSM_OK;
+}
+
 extern "C" {
 
 int gsm_smem_workspace_info(uint64_t n_reads, uint32_t max_len, gsm_workspace_info* out) {

@@ -10,8 +10,10 @@ import numpy as np
 import torch
 
 from . import _capi as capi
+from .ingest import Contigs
 
 RECORD_DTYPE = np.dtype([("read_id", "<u4"), ("qstart", "<u2"), ("qend", "<u2"), ("sa_lo", "<u4"), ("sa_hi", "<u4")])
+HIT_DTYPE = np.dtype([("record", "<u4"), ("contig", "<u4"), ("offset", "<u4"), ("flags", "<u4")])
 _BASES = np.frombuffer(b"ACGT", dtype=np.uint8)
 
 
@@ -208,8 +210,10 @@ class IndexFile:
         return [(n, a) for n, a in sec if a is not None]
 
     @classmethod
-    def save(cls, path, index, lut=None, lut_K=0, rmi=None):
-        """index: DeviceIndex; lut: device table of lut_build (K = lut_K); rmi: RmiParams (None rows / probe table kept if built)."""
+    def save(cls, path, index, lut=None, lut_K=0, rmi=None, contigs=None):
+        """index: DeviceIndex; lut: device table of lut_build (K = lut_K); rmi: RmiParams (None rows / probe table kept if built);
+        contigs: the reference's sequence table (Contigs), stored as a "contigs" header key (names) and a contig_start section.
+        Without contigs the file is exactly what earlier versions wrote."""
         import json as _json
         import zlib
         info = {k: int(getattr(index.info, k)) for k in PackedIndex.FIELDS}
@@ -222,6 +226,11 @@ class IndexFile:
                            "none_rows": [int(x) for x in rmi.none_rows] if rmi.none_rows is not None else None,
                            "max_err": float(getattr(rmi, "max_err", -1.0))}
         secs = cls._sections(index, lut, rmi)
+        if contigs is not None:
+            if contigs.n_bases != int(index.info.n_bases):
+                raise ValueError(f"contigs cover {contigs.n_bases} bases, the index {int(index.info.n_bases)}")
+            head["contigs"] = list(contigs.names)
+            secs.append(("contig_start", contigs.start))
         for n, a in secs:
             head["sections"].append({"name": n, "dtype": str(a.dtype), "shape": list(a.shape), "offset": 0, "nbytes": int(a.nbytes),
                                      "crc32": zlib.crc32(memoryview(np.ascontiguousarray(a)).cast("B")) & 0xFFFFFFFF})
@@ -256,7 +265,8 @@ class IndexFile:
     @classmethod
     def load(cls, path, device="cuda", verify=False):
         """-> (DeviceIndex, lut table or None, lut_K, RmiParams or None).  Sections are memory-mapped and copied to the
-        device; nothing is rebuilt.  verify=True checks every section's CRC-32 first (ValueError on a mismatch)."""
+        device; nothing is rebuilt.  verify=True checks every section's CRC-32 first (ValueError on a mismatch).  The index's
+        `contigs` is the file's sequence table, or None when it was saved without one."""
         import zlib
         require_cuda()
         head = cls.header(path)
@@ -286,6 +296,8 @@ class IndexFile:
         if "seed_table" in arrs:
             index.seed_table, index.seed_K = up("seed_table"), head["seed_K"]
         index._bind()
+        if "contigs" in head:
+            index.set_contigs(Contigs(head["contigs"], np.array(arrs["contig_start"])))
         lut = up("lut")
         rmi = None
         if head["rmi"] is not None:
@@ -306,6 +318,9 @@ class IndexFile:
 class DeviceIndex:
     """The index resident in HBM: two bucket arrays (text / reversed text), optionally the full
     suffix array and the 2-bit text (needed by RMI and by position lookups)."""
+
+    contigs = None          # sequence table (set_contigs); None = the text is one sequence
+    _contig_start = None
 
     def __init__(self, host, device="cuda", with_sa=True, with_text=True):
         """host: a HostIndex (arrays are packed now) or a PackedIndex (arrays loaded from disk)."""
@@ -448,6 +463,19 @@ class DeviceIndex:
             out = torch.empty_like(r)
             capi.check(capi.lib.gsm_locate_sampled_batch(C.byref(self.c), _ptr(self.ssa), self.sa_sample, rows.size, _ptr(r), _ptr(out), _stream()))
         return out.cpu().numpy().view(np.uint32)
+
+    def set_contigs(self, contigs):
+        """Attach the reference's sequence table (ingest.Contigs, e.g. from read_reference): hits are then reported as
+        (sequence, offset).  Its start[n] must equal the index's base count.  None detaches it."""
+        if contigs is None:
+            self.contigs, self._contig_start, self._contigs_c = None, None, None
+            return self
+        if contigs.n_bases != self.n_bases:
+            raise ValueError(f"contigs cover {contigs.n_bases} bases, the index {self.n_bases}")
+        self._contig_start = torch.from_numpy(contigs.start.view(np.int32).copy()).to(self.device)
+        self._contigs_c = capi.DevContigs(len(contigs), self._contig_start.data_ptr())
+        self.contigs = contigs
+        return self
 
     def drop_seed_table(self):
         self.seed_table, self.seed_K = None, 0
@@ -711,6 +739,24 @@ class SmemResult:
         return self.records[self.offsets[i]:self.offsets[i + 1]]
 
 
+class HitResult:
+    """Hits of a record array (HIT_DTYPE: record, contig, offset, flags), in record order and within a record in
+    suffix-array row order, + CSR offsets per record (int64, one entry per record plus one).  Host arrays of their own."""
+
+    def __init__(self, hits, offsets):
+        self.hits, self.offsets = hits, offsets
+
+    def for_record(self, k):
+        return self.hits[self.offsets[k]:self.offsets[k + 1]]
+
+    def for_read(self, result, i):
+        """Hits of read i of `result`, the SmemResult whose records these hits were located from."""
+        return self.hits[self.offsets[result.offsets[i]]:self.offsets[result.offsets[i + 1]]]
+
+    def __len__(self):
+        return len(self.hits)
+
+
 class Engine:
     """Owns the workspace for batches of up to `max_reads` reads of up to `max_len` bases."""
 
@@ -836,6 +882,12 @@ class Engine:
         res = SmemResult(recs, offs, hst.numpy()[:n], n_mems)
         return res if reuse_host_buffers else res.detach()
 
+    def locate_hits(self, max_occ=500, min_len=0, hit_cap=None):
+        """Hits of the records of the batch this engine selected last, located on the device straight from its record
+        buffer (locate_hits has the semantics)."""
+        _, n_rec = self.check_overflow()
+        return _expand_hits(self.index, self.records, n_rec, max_occ, min_len, hit_cap)
+
     def _grow(self):
         dev = self.device
         self.mem_cap = min(self.mem_cap * 4, (1 << 32) - 1)
@@ -880,6 +932,67 @@ def sa_lookup(index: DeviceIndex, rows):
     out = torch.empty_like(r)
     capi.check(capi.lib.gsm_sa_lookup_batch(C.byref(index.c), rows.size, _ptr(r), _ptr(out), _stream()))
     return out.cpu().numpy().view(np.uint32)
+
+
+def locate_hits(index: DeviceIndex, records, max_occ=500, min_len=0, hit_cap=None):
+    """SMEM records (RECORD_DTYPE, e.g. SmemResult.records) -> HitResult: every record's occurrences on the reference as
+    (sequence, offset), BWA's mem_collect_seeds sampling.  A record of len = qend - qstart < min_len has no hits; otherwise
+    min(cnt, max_occ) of its cnt rows (max_occ = 0: all), row lo + k * (cnt // max_occ) for hit k when cnt > max_occ
+    (flag HIT_SAMPLED).  HIT_SPANS flags a match that runs past the end of its sequence.  Sequences: index.contigs, else
+    one sequence.  Positions from the full suffix array when resident, else from the sampled one (build_sampled_sa).
+    The hits are expanded on the device in slices of at most hit_cap hits (default: all at once; never fewer than the
+    largest record's count) and copied to pinned host memory slice by slice."""
+    require_cuda()
+    recs = np.ascontiguousarray(records).view(RECORD_DTYPE).reshape(-1)
+    n_rec = len(recs)
+    if n_rec and int((recs["sa_hi"][recs["sa_hi"] >= recs["sa_lo"]]).max(initial=0)) >= index.n_rows:
+        raise ValueError("a record's interval lies outside the index")
+    dev = torch.from_numpy(recs.view(np.uint8).reshape(-1)).to(index.device) if n_rec else torch.empty(16, dtype=torch.uint8, device=index.device)
+    return _expand_hits(index, dev, n_rec, max_occ, min_len, hit_cap)
+
+
+def _expand_hits(index, recs, n_rec, max_occ, min_len, hit_cap):
+    """gsm_hits_count + gsm_hits_locate over records already on the device (recs: uint8 tensor, n_rec x 16 bytes)."""
+    ssa = getattr(index, "ssa", None)
+    if index.sa is None and ssa is None:
+        raise ValueError("no suffix array on the device: call build_sampled_sa() before dropping it")
+    max_occ, min_len = int(max_occ), int(min_len)
+    if max_occ < 0 or min_len < 0:
+        raise ValueError("max_occ and min_len must be >= 0")
+    with torch.cuda.device(index.device):
+        dev = index.device
+        counts = torch.empty(max(n_rec, 1), dtype=torch.int32, device=dev)
+        off = torch.empty(n_rec + 1, dtype=torch.int64, device=dev)
+        tmp_bytes = C.c_uint64()
+        capi.check(capi.lib.gsm_hits_workspace_info(n_rec, C.byref(tmp_bytes)))
+        tmp = torch.empty(max(int(tmp_bytes.value), 8), dtype=torch.uint8, device=dev)
+        capi.check(capi.lib.gsm_hits_count(_ptr(recs), n_rec, max_occ, min_len, _ptr(counts), _ptr(off), _ptr(tmp), int(tmp_bytes.value), _stream()))
+        offsets = off.cpu().numpy()
+        total = int(offsets[-1])
+        if total == 0:
+            return HitResult(np.zeros(0, HIT_DTYPE), offsets)
+        cap = total if hit_cap is None else max(int(hit_cap), int(np.diff(offsets).max()))
+        cap = min(cap, total)
+        out = torch.empty(cap * 16, dtype=torch.uint8, device=dev)
+        status = torch.zeros(1, dtype=torch.int64, device=dev)
+        host = torch.empty(total * 16, dtype=torch.uint8, pin_memory=True)
+        contigs = C.byref(index._contigs_c) if index.contigs is not None else None
+        ssa_p, sample = (_ptr(ssa), int(index.sa_sample)) if ssa is not None else (C.c_void_p(0), 0)
+        a = 0
+        while a < n_rec:
+            # records [a, b): as many as fit in cap hits (one at least)
+            b = max(int(np.searchsorted(offsets, offsets[a] + cap, side="right")) - 1, a + 1)
+            b = min(b, n_rec)
+            h0, h1 = int(offsets[a]), int(offsets[b])
+            if h1 > h0:
+                capi.check(capi.lib.gsm_hits_locate(C.byref(index.c), ssa_p, sample, contigs, _ptr(recs), _ptr(off), a, b, max_occ, min_len,
+                                                    _ptr(out), cap, _ptr(status), _stream()))
+                host[h0 * 16:h1 * 16].copy_(out[:(h1 - h0) * 16], non_blocking=True)
+            a = b
+        torch.cuda.current_stream().synchronize()
+        if int(status.item()) != 0:
+            raise capi.GsmError(capi.E_CAPACITY, "gsm_hits_locate: hit buffer overflow")
+    return HitResult(host.numpy().view(HIT_DTYPE), offsets)
 
 
 def set_rmi_prefilter(on=True):

@@ -71,6 +71,63 @@ def read_fasta(path):
     return names, seqs
 
 
+class Contigs:
+    """Sequence table of a reference built from several sequences laid end to end (as BWA concatenates them):
+    names[i], start[i] = first base of sequence i in the concatenated text (uint32, n + 1 entries, start[n] = n_bases;
+    empty sequences allowed) and lengths[i] = start[i + 1] - start[i]."""
+
+    def __init__(self, names, start):
+        s = np.asarray(start, np.int64).reshape(-1)
+        names = [str(x) for x in names]
+        if len(names) < 1 or len(s) != len(names) + 1:
+            raise ValueError("Contigs: need at least one sequence and one more start entry than names")
+        if s[0] != 0 or (np.diff(s) < 0).any() or s[-1] >= 1 << 32:
+            raise ValueError("Contigs: start must begin at 0, never decrease and stay below 2^32")
+        self.names = names
+        self.start = s.astype(np.uint32)
+        self.lengths = np.diff(s).astype(np.uint32)
+
+    @classmethod
+    def single(cls, n_bases):
+        """The whole text as one sequence named ""."""
+        return cls([""], [0, int(n_bases)])
+
+    @classmethod
+    def from_lengths(cls, names, lengths):
+        return cls(names, np.concatenate(([0], np.cumsum(np.asarray(lengths, np.int64)))))
+
+    @property
+    def n_bases(self):
+        return int(self.start[-1])
+
+    def __len__(self):
+        return len(self.names)
+
+    def __eq__(self, other):
+        return isinstance(other, Contigs) and self.names == other.names and np.array_equal(self.start, other.start)
+
+    def __repr__(self):
+        return f"Contigs({len(self)} sequences, {self.n_bases} bases)"
+
+
+def read_reference(path):
+    """Multi-record FASTA -> (text, Contigs): text = every record's bases concatenated (uint8 ASCII; pass text.tobytes() to
+    HostIndex.build or DeviceIndex.build_on_device), Contigs = where each record starts.  A character outside ACGT (N, lower
+    case, IUPAC codes) raises BaseError, as building an index from it would."""
+    from .engine import BaseError
+    names, seqs = read_fasta(path)
+    if not names:
+        raise ValueError(f"{path}: no sequence")
+    contigs = Contigs.from_lengths(names, [len(q) for q in seqs])
+    text = np.concatenate(seqs) if seqs else np.zeros(0, np.uint8)
+    bad = np.flatnonzero(~_VALID[text])
+    if len(bad):
+        p = int(bad[0])
+        c = int(np.searchsorted(contigs.start, p, side="right")) - 1
+        raise BaseError(f"{path}: sequence {names[c]!r} holds {chr(text[p])!r} at offset {p - int(contigs.start[c])}: only ACGT can be indexed")
+    return text, contigs
+
+
 def read_fastq(path, n_policy="error", pin=True, threads=0):
     """4-line FASTQ -> (bases uint8 (pinned when a GPU is present), base_off int64[n+1], dropped read indices).
     The file is cut into records and its sequence lines are gathered by the library's multi-threaded scanner

@@ -419,6 +419,48 @@ int gsm_device_l2_fetch_granularity(int32_t set_bytes, uint32_t* current);
 const char* gsm_last_error(void);
 int gsm_version(void);
 
+/* ------------------------------------------------------------------ hits: records -> reference positions
+ * Expands SMEM records into capped occurrence positions in per-sequence coordinates: ExactMatch.exact_match /
+ * get_positions (ExactMatch.py:174-199) and the positions LUT.lut stores per k-mer (LUT.py:33-35), for a whole batch.
+ *
+ * Record r = {read_id, qstart, qend, lo, hi}: cnt = hi - lo + 1, len = qend - qstart.  n_hits(r) = 0 if len < min_len,
+ * else min(cnt, max_occ) (max_occ == 0: no cap).  Hit k (0 <= k < n_hits) is row lo + k * step, step = cnt / max_occ
+ * when cnt > max_occ, else 1 (BWA's mem_collect_seeds rule: hits in suffix-array row order).  Its 0-based text position
+ * p = suffix_array[row] - 1 lies in sequence c = upper_bound(start, p) - 1 at offset p - start[c].
+ *
+ * The reference is the concatenation of n sequences; start (device, n + 1 entries, non-decreasing, start[0] = 0,
+ * start[n] = n_bases; empty sequences allowed) gives where each begins.  A NULL gsm_dev_contigs = one sequence. */
+typedef struct {
+    uint64_t n;             /* sequences */
+    const uint32_t* start;  /* device, n + 1 entries */
+} gsm_dev_contigs;
+
+#define GSM_HIT_SPANS 1u   /* offset + len > length of the sequence: the match runs into the next sequence */
+#define GSM_HIT_SAMPLED 2u /* cnt > max_occ: the hits are an evenly spaced sample of the interval */
+
+typedef struct {
+    uint32_t record; /* index of the record in the array passed in */
+    uint32_t contig;
+    uint32_t offset; /* 0-based, in the sequence */
+    uint32_t flags;  /* GSM_HIT_* */
+} gsm_hit;
+
+/* Bytes of device scratch gsm_hits_count needs for n_recs records (host arithmetic, no device needed). */
+int gsm_hits_workspace_info(uint64_t n_recs, uint64_t* scan_tmp_bytes);
+
+/* Phase 1: counts_u32[r] = n_hits(r) and hit_off_u64 (n_recs + 1 entries) = their exclusive scan, hit_off_u64[n_recs] =
+ * the total.  recs, counts_u32, hit_off_u64 and scan_tmp are device memory.  Asynchronous on stream. */
+int gsm_hits_count(const gsm_record* recs, uint64_t n_recs, uint32_t max_occ, uint32_t min_len, uint32_t* counts_u32,
+                   uint64_t* hit_off_u64, void* scan_tmp, uint64_t scan_tmp_bytes, void* stream);
+
+/* Phase 2: the hits of records [rec_begin, rec_end), hit h at out[h - hit_off[rec_begin]] (device, out_cap entries).
+ * Positions come from idx->sa when it is set, else from ssa (gsm_sa_sample_build, every `sample`-th row) by LF walks; with
+ * neither, GSM_E_INVALID.  max_occ / min_len must be those given to gsm_hits_count.  Nothing is written at or past out_cap;
+ * if the range holds more hits, bit 0 of *status8 (device uint64) is set.  Asynchronous on stream. */
+int gsm_hits_locate(const gsm_dev_index* idx, const uint32_t* ssa, uint32_t sample, const gsm_dev_contigs* contigs,
+                    const gsm_record* recs, const uint64_t* hit_off, uint64_t rec_begin, uint64_t rec_end, uint32_t max_occ,
+                    uint32_t min_len, gsm_hit* out, uint64_t out_cap, uint64_t* status8, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
