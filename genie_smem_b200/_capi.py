@@ -83,6 +83,7 @@ EXPORTS = {
     "gsm_pack_reads_scattered_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p,
                                                   C.c_void_p]),
     "gsm_pack_reads_device_check": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "gsm_reads_both_strands_device": (C.c_int, [C.POINTER(DevReads), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsm_smem_workspace_info": (C.c_int, [C.c_uint64, C.c_uint32, C.POINTER(WorkspaceInfo)]),
     "gsm_backsearch_batch": (C.c_int, [C.POINTER(DevIndex), C.POINTER(DevReads), C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsm_backsearch_add_one_batch": (C.c_int, [C.POINTER(DevIndex), C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -10,6 +10,7 @@
 
 #include "../../include/genie_smem.h"
 #include "host_common.hpp"
+#include "strand_logic.cuh"
 
 namespace gsm {
 
@@ -203,6 +204,49 @@ __global__ void __launch_bounds__(256) k_pack_reads_scattered(const uint8_t* bas
     }
 }
 
+// Strand-doubled batch: read r of the input -> slot 2r (the read) and slot 2r+1 (its reverse complement), one warp per
+// read, one lane per output word pair (strand_logic.cuh).  Chunk offsets are rebased to the view's first read: slot 2r
+// starts at 2 (c[r] - c[0]), slot 2r+1 right after it.  Thread 0 also writes the closing offset and zeroes the pad chunk.
+__global__ void __launch_bounds__(256) k_both_strands(const uint32_t* __restrict__ src, const uint32_t* __restrict__ chunk_off,
+                                                      const uint32_t* __restrict__ len, uint64_t n_reads, uint32_t* __restrict__ dst,
+                                                      uint32_t* __restrict__ chunk_off_out, uint32_t* __restrict__ len_out) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const uint64_t n_warps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
+    const uint32_t c0 = __ldg(chunk_off);
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        const uint32_t end = 2u * (__ldg(chunk_off + n_reads) - c0);
+        chunk_off_out[2 * n_reads] = end;
+        reinterpret_cast<uint4*>(dst)[end] = make_uint4(0u, 0u, 0u, 0u);
+    }
+    for (uint64_t r = warp0; r < n_reads; r += n_warps) {
+        const uint32_t a = __ldg(chunk_off + r) - c0, nch = __ldg(chunk_off + r + 1) - c0 - a;
+        const uint32_t L0 = __ldg(len + r);
+        const uint32_t L = min(L0, nch * 64u);              // never read past the read's own chunks
+        if (lane == 0) {
+            chunk_off_out[2 * r] = 2u * a;
+            chunk_off_out[2 * r + 1] = 2u * a + nch;
+            len_out[2 * r] = L0;
+            len_out[2 * r + 1] = L0;
+        }
+        const uint32_t* s = src + (uint64_t)(a + c0) * 4u;
+        uint32_t* fwd = dst + (uint64_t)a * 8u;
+        uint32_t* rc = fwd + (uint64_t)nch * 4u;
+        for (uint32_t w = lane; w < nch * 4u; w += 32u) {
+            const uint32_t m = strand_word_mask(L, w);
+            fwd[w] = m ? __ldg(s + w) & m : 0u;
+            StrandSrc q;
+            uint32_t v = 0u;
+            if (strand_rc_src(L, w, &q)) {
+                const uint32_t hi = q.q >= 0 ? __ldg(s + q.q) : 0u;
+                const uint32_t lo = q.sh ? __ldg(s + q.q + 1) : 0u;
+                v = strand_rc_word(hi, lo, q.sh, L, w);
+            }
+            rc[w] = v;
+        }
+    }
+}
+
 }  // namespace
 }  // namespace gsm
 
@@ -280,6 +324,22 @@ int gsm_pack_reads_scattered_device(const void* bases, const uint64_t* seq_start
     const unsigned grid = (unsigned)std::min<uint64_t>((n_reads + 7) / 8, 148ull * 32);
     k_pack_reads_scattered<<<grid, 256, 0, st>>>((const uint8_t*)bases, (const unsigned long long*)seq_start, seq_len, chunk_off, n_reads, (int)ascii,
                                                  (uint32_t*)packed, (unsigned long long*)scratch8);
+    GSM_CUDA(cudaGetLastError());
+    return GSM_OK;
+}
+
+int gsm_reads_both_strands_device(const gsm_dev_reads* in, void* packed_out, uint32_t* chunk_off_out, uint32_t* len_out, void* stream) {
+    if (!in || !packed_out || !chunk_off_out || !len_out || !in->packed || !in->chunk_off || (in->n_reads && !in->len))
+        return fail(GSM_E_INVALID, "gsm_reads_both_strands_device: null");
+    // the doubled offsets are at most 2 * n * ceil(max_len / 64) chunks
+    const uint64_t n = in->n_reads;
+    if (n >= (1ull << 31) || 2ull * n * (((uint64_t)in->max_len + 63) / 64) >= (1ull << 32))
+        return fail(GSM_E_CAPACITY, "gsm_reads_both_strands_device: the doubled chunk offsets do not fit in 32 bits");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(GSM_E_NODEVICE, "no CUDA device");
+    const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((n + 7) / 8, 148ull * 32));
+    k_both_strands<<<grid, 256, 0, (cudaStream_t)stream>>>((const uint32_t*)in->packed, in->chunk_off, in->len, n, (uint32_t*)packed_out,
+                                                           chunk_off_out, len_out);
     GSM_CUDA(cudaGetLastError());
     return GSM_OK;
 }

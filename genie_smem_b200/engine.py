@@ -606,6 +606,37 @@ class ReadBatch:
         r.max_len, r.read_id_base = self.max_len, self.read_id_base
         return r
 
+    def both_strands(self):
+        """The strand-doubled batch, built on the device (gsm_reads_both_strands_device): 2n reads, slot 2i = read i as
+        given, slot 2i+1 = its reverse complement, read_id_base = 2 * self.read_id_base, so that a record's read_id >> 1
+        is the read and read_id & 1 its strand.  A batch that only lives on the host is copied to the current CUDA
+        device first.  Raises ValueError when the doubled read ids would reach 2^32."""
+        require_cuda()
+        _check_doubled_ids(self.read_id_base, self.n)
+        if self.packed is None:
+            self.to(torch.device("cuda"))
+        dev = self.packed.device
+        n = self.n
+        co = self.chunk_off_host if self.chunk_off_host is not None else self.chunk_off.cpu().numpy().view(np.uint32)
+        c = co[: n + 1].astype(np.int64) - int(co[0])
+        coff = np.empty(2 * n + 1, np.int64)
+        coff[0::2], coff[1::2] = 2 * c, c[:-1] + c[1:]
+        if coff[-1] >= 1 << 32:
+            raise capi.GsmError(capi.E_CAPACITY, "strand-doubled batch too large for 32-bit chunk offsets")
+        lens = self.len_host if self.len_host is not None and len(self.len_host) == n else self.len[:n].cpu().numpy().view(np.uint32)
+        out = ReadBatch(None, coff.astype(np.uint32), np.repeat(np.asarray(lens, np.uint32), 2), self.max_len, 2 * self.read_id_base)
+        with torch.cuda.device(dev):
+            out.packed = torch.empty(int(coff[-1]) * 16 + 16, dtype=torch.uint8, device=dev)
+            out.chunk_off = torch.empty(2 * n + 1, dtype=torch.int32, device=dev)
+            out.len = torch.empty(max(2 * n, 1), dtype=torch.int32, device=dev)[: 2 * n]
+            capi.check(capi.lib.gsm_reads_both_strands_device(C.byref(self.cstruct()), _ptr(out.packed), _ptr(out.chunk_off), _ptr(out.len), _stream()))
+        return out
+
+
+def _check_doubled_ids(read_id_base, n):
+    if 2 * (int(read_id_base) + int(n)) >= 1 << 32:
+        raise ValueError(f"strands=2: read ids 2 * ({read_id_base} + {n}) do not fit in 32 bits")
+
 
 class RmiParams:
     """(coef, intercept) per linear model of an RMI (reference SMEM/RMI.py), on the device."""
@@ -724,19 +755,51 @@ class RmiParams:
 class SmemResult:
     """Records of one batch in (read, emission) order + CSR offsets per read.
 
+    strands = 2 (an engine built with strands=2): the batch was searched strand-doubled, so offsets, status and the records'
+    read ids are per SLOT -- slot 2i is read i as given, slot 2i+1 its reverse complement, read_id = 2 * (read_id_base + i)
+    + strand, and a strand-1 record's qstart / qend are in the reverse complement's coordinates.  `lengths` then holds the
+    length of every read (uint32), which read_coords() needs.
+
     Lifetime: by default the arrays are the caller's own copies.  With reuse_host_buffers=True (Engine.run /
     PipelinedEngine.run*) they are VIEWS of the engine's pinned staging buffers and are overwritten by that engine's
     next run -- the zero-copy mode bench.py times; copy what you keep."""
 
-    def __init__(self, records, offsets, status, n_mems):
+    def __init__(self, records, offsets, status, n_mems, strands=1, lengths=None):
         self.records, self.offsets, self.status, self.n_mems = records, offsets, status, n_mems
+        self.strands, self.lengths = strands, lengths
 
     def detach(self):
         self.records, self.offsets, self.status = self.records.copy(), self.offsets.copy(), self.status.copy()
+        if self.lengths is not None:
+            self.lengths = self.lengths.copy()
         return self
 
-    def for_read(self, i):
-        return self.records[self.offsets[i]:self.offsets[i + 1]]
+    def _slots(self, i, strand):
+        """Slot range [a, b) of read i: both strands (strand None) or one."""
+        if strand not in (None, 0, 1) or (self.strands == 1 and strand == 1):
+            raise ValueError(f"strand must be None, 0{' or 1' if self.strands == 2 else ''}")
+        if self.strands == 1:
+            return i, i + 1
+        return (2 * i, 2 * i + 2) if strand is None else (2 * i + strand, 2 * i + strand + 1)
+
+    def for_read(self, i, strand=None):
+        """Records of read i; with strands = 2 those of both its slots (strand None, slot 2i first) or of one strand."""
+        a, b = self._slots(i, strand)
+        return self.records[self.offsets[a]:self.offsets[b]]
+
+    def read_coords(self):
+        """Per-record arrays in the ORIGINAL read's orientation: `read` (read_id >> 1 with strands = 2, else read_id),
+        `strand` (0 / 1), and the matched bases read[qbeg:qend] -- for a strand-1 record qbeg = L - qend, qend = L - qstart,
+        the same bases seen on the reverse strand."""
+        rid = self.records["read_id"]
+        qs, qe = self.records["qstart"].astype(np.uint32), self.records["qend"].astype(np.uint32)
+        if self.strands == 1:
+            return {"read": rid.copy(), "strand": np.zeros(len(rid), np.uint8), "qbeg": qs, "qend": qe}
+        slot = np.repeat(np.arange(len(self.offsets) - 1), np.diff(self.offsets))
+        strand = (rid & 1).astype(np.uint8)
+        L = np.asarray(self.lengths, np.uint32)[slot >> 1]
+        rev = strand == 1
+        return {"read": rid >> 1, "strand": strand, "qbeg": np.where(rev, L - qe, qs), "qend": np.where(rev, L - qs, qe)}
 
 
 class HitResult:
@@ -749,27 +812,38 @@ class HitResult:
     def for_record(self, k):
         return self.hits[self.offsets[k]:self.offsets[k + 1]]
 
-    def for_read(self, result, i):
-        """Hits of read i of `result`, the SmemResult whose records these hits were located from."""
-        return self.hits[self.offsets[result.offsets[i]]:self.offsets[result.offsets[i + 1]]]
+    def for_read(self, result, i, strand=None):
+        """Hits of read i of `result`, the SmemResult whose records these hits were located from (strand as in
+        SmemResult.for_read)."""
+        a, b = result._slots(i, strand)
+        return self.hits[self.offsets[result.offsets[a]]:self.offsets[result.offsets[b]]]
 
     def __len__(self):
         return len(self.hits)
 
 
 class Engine:
-    """Owns the workspace for batches of up to `max_reads` reads of up to `max_len` bases."""
+    """Owns the workspace for batches of up to `max_reads` reads of up to `max_len` bases.
 
-    def __init__(self, index: DeviceIndex, max_reads, max_len, mems_per_read=24, recs_per_read=16):
+    strands = 2: run() searches every read and its reverse complement in one batch.  The batch is strand-doubled on the
+    device (ReadBatch.both_strands: slot 2i = read i, slot 2i+1 = its reverse complement) into buffers of this engine,
+    so the workspace holds 2 * max_reads slots, and the result is per slot (SmemResult.strands = 2).  sweep / select /
+    launch take the batch they are given, doubled or not."""
+
+    def __init__(self, index: DeviceIndex, max_reads, max_len, mems_per_read=24, recs_per_read=16, strands=1):
         require_cuda()
+        if strands not in (1, 2):
+            raise ValueError("strands must be 1 or 2")
         self.index = index
         self.device = index.device
         self.max_reads, self.max_len = int(max_reads), int(max_len)
+        self.strands = int(strands)
+        self.slots = self.strands * self.max_reads
         wi = capi.WorkspaceInfo()
-        capi.check(capi.lib.gsm_smem_workspace_info(self.max_reads, self.max_len, C.byref(wi)))
+        capi.check(capi.lib.gsm_smem_workspace_info(self.slots, self.max_len, C.byref(wi)))
         self.grid = (int(wi.grid_blocks), int(wi.block_threads))
         dev = self.device
-        n = max(self.max_reads, 1)
+        n = max(self.slots, 1)
         self.mem_cap = min(max(n * mems_per_read, 4096), (1 << 32) - 1)
         self.rec_cap = min(max(n * recs_per_read, 4096), (1 << 32) - 1)
         self.mem_pool = torch.empty(self.mem_cap * 16, dtype=torch.uint8, device=dev)
@@ -796,10 +870,27 @@ class Engine:
         self.kernel_launches = 0
         self._pin = {}
         self.last_d2h_bytes = 0
+        if self.strands == 2:                     # the strand-doubled batch: 2 * max_reads reads of up to max_len bases
+            m = max(self.max_reads, 1)
+            self.ds_packed = torch.empty(2 * m * ((self.max_len + 63) // 64) * 16 + 16, dtype=torch.uint8, device=dev)
+            self.ds_chunk_off = torch.empty(2 * m + 1, dtype=torch.int32, device=dev)
+            self.ds_len = torch.empty(2 * m, dtype=torch.int32, device=dev)
+
+    def _both_strands(self, reads):
+        """Strand-double reads (a ReadBatch or a view of one on the device) into this engine's buffers, on the current
+        stream; -> the doubled batch as a view, read_id_base and lo doubled."""
+        if reads.n > self.max_reads or reads.max_len > self.max_len:
+            raise ValueError("batch exceeds the engine's workspace")
+        _check_doubled_ids(reads.read_id_base, reads.n)
+        capi.check(capi.lib.gsm_reads_both_strands_device(C.byref(reads.cstruct()), _ptr(self.ds_packed), _ptr(self.ds_chunk_off),
+                                                          _ptr(self.ds_len), _stream()))
+        self.kernel_launches += 1
+        return _ChunkView(self.ds_packed, self.ds_chunk_off, self.ds_len, 2 * reads.n, reads.max_len, 2 * reads.read_id_base,
+                          2 * getattr(reads, "lo", 0))
 
     # -- device-resident phases: kernels only (bench.py times these as `value`)
     def _check_batch(self, reads):
-        if reads.n > self.max_reads or reads.max_len > self.max_len:
+        if reads.n > self.slots or reads.max_len > self.max_len:
             raise ValueError("batch exceeds the engine's workspace")
         self._reads_c = reads.cstruct()
         return self._reads_c
@@ -813,6 +904,8 @@ class Engine:
     def select(self, method, reads: ReadBatch, min_len=1, K=0, lut=None, rmi: RmiParams = None, gatherer=None):
         """k_select + scan + ordered write: the reference's records for one method, in (read, emission) order -- into
         this engine's `records` buffer, or with a sharding.RecordGatherer straight into the gathering rank's HBM."""
+        if gatherer is not None and self.strands == 2:
+            raise ValueError("strands=2 does not support a gatherer")
         r = self._check_batch(reads)
         capi.check(capi.lib.gsm_smem_select(method, C.byref(self.index.c), C.byref(r), int(min_len), int(K), _ptr(lut),
                                             C.byref(rmi.c) if rmi is not None else None, C.byref(self.ws), _stream()))
@@ -858,7 +951,11 @@ class Engine:
 
     # -- end-to-end step: host reads in (H2D), host records out (D2H)
     def run(self, method, reads: ReadBatch, min_len=1, K=0, lut=None, rmi: RmiParams = None, grow=True, reuse_host_buffers=False):
+        """Host reads in (H2D), host records out (D2H).  With strands=2 the batch is strand-doubled on the device first and
+        the result is per slot (SmemResult.strands = 2)."""
         reads.to(self.device, non_blocking=True)
+        if self.strands == 2:
+            reads = self._both_strands(reads)
         while True:
             self.launch(method, reads, min_len, K, lut, rmi)
             try:
@@ -875,11 +972,18 @@ class Engine:
         hrec[: n_rec * 16].copy_(self.records[: n_rec * 16], non_blocking=True)
         hoff[: (n + 1) * 8].copy_(self.rec_off[: n + 1].view(torch.uint8), non_blocking=True)
         hst[:n].copy_(self.read_status[:n], non_blocking=True)
+        lengths = None
+        if self.strands == 2:
+            hlen = self._pinned("len", max(n, 1) * 4)
+            hlen[: n * 4].copy_(self.ds_len[:n].view(torch.uint8), non_blocking=True)
         torch.cuda.current_stream().synchronize()
         self.last_d2h_bytes = n_rec * 16 + (n + 1) * 8 + n + 64
+        if self.strands == 2:
+            lengths = hlen.numpy()[: n * 4].view(np.uint32)[0::2]
+            self.last_d2h_bytes += n * 4
         recs = hrec.numpy()[: n_rec * 16].view(RECORD_DTYPE)
         offs = hoff.numpy()[: (n + 1) * 8].view(np.int64)
-        res = SmemResult(recs, offs, hst.numpy()[:n], n_mems)
+        res = SmemResult(recs, offs, hst.numpy()[:n], n_mems, self.strands, lengths)
         return res if reuse_host_buffers else res.detach()
 
     def locate_hits(self, max_occ=500, min_len=0, hit_cap=None):
@@ -1109,14 +1213,20 @@ class PipelinedEngine:
       compute   [2-bit packing,] sweep, select, scan, gather of chunk i, in order, alternating between two workspaces,
       copy-out  records / offsets / status of chunk i to pinned host memory as soon as its record count is known.
     The compute stream only waits for chunk i's H2D and for the D2H that frees its workspace (chunk i-2), so neither
-    copy direction ever sits between two sweeps.  Inputs must be pinned."""
+    copy direction ever sits between two sweeps.  Inputs must be pinned.
 
-    def __init__(self, index: DeviceIndex, max_reads, max_len, n_chunks=8, mems_per_read=24, recs_per_read=16):
+    strands = 2: every chunk is strand-doubled on the compute stream right after packing (Engine strands=2: each workspace
+    holds 2 * chunk_reads slots and its own doubled-batch buffers), and the result is per slot (SmemResult.strands = 2)."""
+
+    def __init__(self, index: DeviceIndex, max_reads, max_len, n_chunks=8, mems_per_read=24, recs_per_read=16, strands=1):
         require_cuda()
+        if strands not in (1, 2):
+            raise ValueError("strands must be 1 or 2")
         self.index, self.device = index, index.device
+        self.strands = int(strands)
         self.n_chunks = max(2, int(n_chunks))
         self.chunk_reads = (int(max_reads) + self.n_chunks - 1) // self.n_chunks
-        self.engines = [Engine(index, self.chunk_reads, max_len, mems_per_read, recs_per_read) for _ in range(2)]
+        self.engines = [Engine(index, self.chunk_reads, max_len, mems_per_read, recs_per_read, self.strands) for _ in range(2)]
         self.s_in, self.s_comp, self.s_out = (torch.cuda.Stream(device=self.device) for _ in range(3))
         self.max_reads, self.max_len = int(max_reads), int(max_len)
         self._dev = {}
@@ -1160,6 +1270,7 @@ class PipelinedEngine:
     def run(self, method, reads: ReadBatch, min_len=1, K=0, lut=None, rmi: RmiParams = None, reuse_host_buffers=False, gatherer=None):
         """Packed host reads in (pinned), host records out -- or, with a sharding.RecordGatherer, records written straight
         into the gathering rank's HBM (the result then carries offsets and status only)."""
+        self._check_gatherer(gatherer)
         n = reads.n
         if n > self.max_reads or reads.max_len > self.max_len:
             raise ValueError("batch exceeds the engine's workspace")
@@ -1187,6 +1298,7 @@ class PipelinedEngine:
         (what a FASTQ parser hands over).  Each chunk crosses PCIe as 1 byte/base and is 2-bit packed on the GPU
         (gsm_pack_reads_device) right before its sweep.  Raises BaseError if a read holds a non-ACGT character
         (the reference's KeyError, ExactMatch.py:139)."""
+        self._check_gatherer(gatherer)
         read_len = int(read_len)
         n = bases.numel() // read_len
         if n > self.max_reads or read_len > self.max_len:
@@ -1303,19 +1415,27 @@ class PipelinedEngine:
         res = self._run_chunks(method, self.max_reads, copy_in, prep, min_len, K, lut, rmi, None, dynamic_chunks=n_ch)
         return res if reuse_host_buffers else res.detach()
 
+    def _check_gatherer(self, gatherer):
+        if gatherer is not None and self.strands == 2:
+            raise ValueError("strands=2 does not support a gatherer")
+
     def _run_chunks(self, method, n, copy_in, prep, min_len, K, lut, rmi, gatherer=None, dynamic_chunks=0):
         """dynamic_chunks = 0: the batch of n reads is cut by _chunk_bounds; copy_in(lo, hi) / prep(lo, hi) take read ranges.
         dynamic_chunks = k: k chunks whose read counts are only known once they are prepared (FASTQ bytes): copy_in(i) /
-        prep(i) take the chunk index, prep's view carries .lo / .hi, and n is the capacity the outputs are sized for."""
+        prep(i) take the chunk index, prep's view carries .lo / .hi, and n is the capacity the outputs are sized for.
+        With strands = 2 each prepared chunk is strand-doubled and everything downstream is in slot space (2 lo .. 2 hi)."""
         if dynamic_chunks:
             bounds, n_ch = None, int(dynamic_chunks)
         else:
             bounds = self._chunk_bounds(n)
             n_ch = len(bounds) - 1
+        ns = self.strands
+        n_cap = n * ns                                          # slots the outputs are sized for
         est = self.engines[0].rec_cap * 16
         out_rec = self._buf(self._pin, "rec", max(est, 1 << 20), True)
-        out_off = self._buf(self._pin, "off", (n + 1) * 8, True)
-        out_st = self._buf(self._pin, "st", max(n, 1), True)
+        out_off = self._buf(self._pin, "off", (n_cap + 1) * 8, True)
+        out_st = self._buf(self._pin, "st", max(n_cap, 1), True)
+        out_len = self._buf(self._pin, "len", max(n_cap, 1) * 4, True) if ns == 2 else None
         start_ev = torch.cuda.Event()
         start_ev.record(torch.cuda.current_stream())
         ev_in = []
@@ -1361,6 +1481,8 @@ class PipelinedEngine:
                     eng.rec_off[: hi - lo].add_(rec_total)
                 out_off[lo * 8:hi * 8].copy_(eng.rec_off[: hi - lo].view(torch.uint8), non_blocking=True)
                 out_st[lo:hi].copy_(eng.read_status[: hi - lo], non_blocking=True)
+                if out_len is not None:
+                    out_len[lo * 4:hi * 4].copy_(eng.ds_len[: hi - lo].view(torch.uint8), non_blocking=True)
                 d = torch.cuda.Event()
                 d.record(self.s_out)
                 ev_out[i] = d
@@ -1385,6 +1507,9 @@ class PipelinedEngine:
                 else:
                     lo, hi = bounds[i], bounds[i + 1]
                     view = prep(lo, hi)
+                if ns == 2:
+                    view = eng._both_strands(view)
+                    lo, hi = 2 * lo, 2 * hi
                 n_seen = max(n_seen, hi)
                 eng.launch(method, view, min_len, K, lut, rmi, gatherer)
                 self._cnt_pin[e].copy_(eng.counters, non_blocking=True)
@@ -1396,11 +1521,14 @@ class PipelinedEngine:
         self.s_out.synchronize()
         self.s_comp.synchronize()
         torch.cuda.current_stream().wait_stream(self.s_out)
-        if dynamic_chunks:
-            n = n_seen
+        n = n_seen if dynamic_chunks else n_cap                 # slots
         offs = out_off.numpy()[: (n + 1) * 8].view(np.int64)
         offs[n] = rec_total
         self.kernel_launches = sum(e.kernel_launches for e in self.engines) + self.pack_launches
         self.last_d2h_bytes = (rec_total * 16 if gatherer is None else 0) + (n + 1) * 8 + n + 64 * len(chunk_rec)
         recs = out_rec.numpy()[: (rec_total if gatherer is None else 0) * 16].view(RECORD_DTYPE)
-        return SmemResult(recs, offs, out_st.numpy()[:n], mems_total)
+        lengths = None
+        if out_len is not None:
+            lengths = out_len.numpy()[: n * 4].view(np.uint32)[0::2]
+            self.last_d2h_bytes += n * 4
+        return SmemResult(recs, offs, out_st.numpy()[:n], mems_total, ns, lengths)

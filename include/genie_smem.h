@@ -192,6 +192,25 @@ typedef struct {
     uint32_t read_id_base;     /* added to the read index in emitted records (rank sharding) */
 } gsm_dev_reads;
 
+/* Strand-doubled batch, built ON THE GPU: the n reads of `in` become 2n slots, interleaved -- slot 2i is read i as given,
+ * slot 2i+1 its reverse complement (base k = 3 - base[L-1-k] in the A=0 C=1 G=2 T=3 codes).  Run the SMEM entry points
+ * on the doubled batch with read_id_base = 2 * (the original read_id_base): a record's read_id is then
+ * 2 * (read_id_base + i) + strand, so read_id >> 1 is the read and read_id & 1 the strand.  Slot 2i gets exactly the
+ * records of read i in every field but read_id; slot 2i+1 gets what the method gives for the reverse-complement string,
+ * with qstart / qend in ITS coordinates (read[L-qend : L-qstart] on the reverse strand); a palindromic read gets the same
+ * records on both strands.  A hit of a strand-1 record at (contig, offset) means RC(read)[qstart:qend] occurs on the
+ * forward strand there: the hit entry points do not change.
+ *   in:            reads in->packed, in->chunk_off (n+1) and in->len (n); may be a view of reads [lo, hi) with
+ *                  chunk_off[0] != 0.  in->max_len bounds the lengths.
+ *   chunk_off_out: 2n+1 entries starting at 0: [2r] = 2 (c[r] - c[0]), [2r+1] = (c[r] - c[0]) + (c[r+1] - c[0]).
+ *   len_out:       2n entries.
+ *   packed_out:    2 (c[n] - c[0]) * 16 + 16 bytes; pad bits and the pad chunk are zero, so the output is byte-identical
+ *                  to gsm_pack_reads of the interleaved strings [r0, rc(r0), r1, rc(r1), ...].
+ * GSM_E_INVALID for a null pointer, GSM_E_CAPACITY when 2 n ceil(max_len / 64) chunks would not fit in 32 bits.
+ * Asynchronous on `stream`. */
+int gsm_reads_both_strands_device(const gsm_dev_reads* in, void* packed_out, uint32_t* chunk_off_out, uint32_t* len_out,
+                                  void* stream);
+
 /* One emitted SMEM, before the reference's dict collapses duplicate strings.  16 bytes. */
 typedef struct {
     uint32_t read_id;
