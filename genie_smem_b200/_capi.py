@@ -61,6 +61,14 @@ class Hit(C.Structure):
 
 HIT_SPANS, HIT_SAMPLED = 1, 2
 
+
+class Chain(C.Structure):
+    _fields_ = [("slot", C.c_uint32), ("contig", C.c_uint32), ("rbeg", C.c_uint32), ("rend", C.c_uint32), ("q", C.c_uint32),
+                ("weight", C.c_uint32), ("n_seeds", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+CHAIN_NONE, CHAIN_CONTAINED = 0xFFFFFFFF, 0x80000000
+
 EXPORTS = {
     # name: (restype, argtypes)
     "gsm_index_build": (C.c_int, [C.c_char_p, C.c_uint64, C.c_uint32, C.POINTER(C.c_void_p)]),
@@ -129,6 +137,11 @@ EXPORTS = {
     "gsm_hits_count": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "gsm_hits_locate": (C.c_int, [C.POINTER(DevIndex), C.c_void_p, C.c_uint32, C.POINTER(DevContigs), C.c_void_p, C.c_void_p, C.c_uint64,
                                   C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
+    "gsm_chains_workspace_info": (C.c_int, [C.c_uint64, C.c_uint64, C.POINTER(C.c_uint64)]),
+    "gsm_chain_seeds": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p,
+                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
+    "gsm_chains_collect": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64,
+                                     C.c_void_p, C.c_void_p]),
 }
 
 

@@ -11,8 +11,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "_obj")
 LIB = os.path.join(HERE, "libgenie_smem.so")
-SOURCES = ["kernels.cu", "index_device.cu", "ingest.cu", "comm.cu", "hits.cu", "index_host.cpp", "ingest_host.cpp"]
-HEADERS = ["fm_core.cuh", "sweep_logic.cuh", "sweep_device.cuh", "select_logic.cuh", "hits_logic.cuh", "strand_logic.cuh", "host_common.hpp", "../../include/genie_smem.h"]
+SOURCES = ["kernels.cu", "index_device.cu", "ingest.cu", "comm.cu", "hits.cu", "chains.cu", "index_host.cpp", "ingest_host.cpp"]
+HEADERS = ["fm_core.cuh", "sweep_logic.cuh", "sweep_device.cuh", "select_logic.cuh", "hits_logic.cuh", "strand_logic.cuh", "chain_logic.cuh", "host_common.hpp",
+           "../../include/genie_smem.h"]
 FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
          "-Xcompiler", "-fPIC,-O3,-fno-strict-aliasing", "-Xptxas", "-v"]
 

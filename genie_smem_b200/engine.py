@@ -14,6 +14,8 @@ from .ingest import Contigs
 
 RECORD_DTYPE = np.dtype([("read_id", "<u4"), ("qstart", "<u2"), ("qend", "<u2"), ("sa_lo", "<u4"), ("sa_hi", "<u4")])
 HIT_DTYPE = np.dtype([("record", "<u4"), ("contig", "<u4"), ("offset", "<u4"), ("flags", "<u4")])
+CHAIN_DTYPE = np.dtype([("slot", "<u4"), ("contig", "<u4"), ("rbeg", "<u4"), ("rend", "<u4"), ("q", "<u4"), ("weight", "<u4"),
+                        ("n_seeds", "<u4"), ("reserved", "<u4")])
 _BASES = np.frombuffer(b"ACGT", dtype=np.uint8)
 
 
@@ -822,6 +824,57 @@ class HitResult:
         return len(self.hits)
 
 
+class ChainResult:
+    """BWA-MEM's co-linear chains of every slot (chain_seeds has the semantics): `chains` (CHAIN_DTYPE) in slot order, within
+    a slot in (contig, rbeg) order; `offsets` (int64, one entry per slot plus one); `hits`, the HitResult of the slots'
+    records; `hit_chain` (u32 per hit): the index within its slot of the chain the hit belongs to, | CHAIN_CONTAINED when it
+    was contained in that chain rather than appended, CHAIN_NONE for a spanning hit; `rec_offsets`: the records of each slot
+    (the SmemResult's offsets).  strands / lengths as in SmemResult.  Host arrays of their own."""
+
+    def __init__(self, chains, offsets, hits, hit_chain, rec_offsets, strands=1, lengths=None):
+        self.chains, self.offsets, self.hits, self.hit_chain = chains, offsets, hits, hit_chain
+        self.rec_offsets, self.strands, self.lengths = rec_offsets, strands, lengths
+
+    def __len__(self):
+        return len(self.chains)
+
+    def for_read(self, i, strand=None):
+        """Chains of read i: with strands = 2 those of both its slots (strand None, slot 2i first) or of one strand."""
+        a, b = SmemResult._slots(self, i, strand)
+        return self.chains[self.offsets[a]:self.offsets[b]]
+
+    def seeds(self, k):
+        """Indices into hits.hits of the member seeds of chain k, in member order (contained seeds are not members)."""
+        s = int(self.chains["slot"][k])
+        a, b = int(self.hits.offsets[self.rec_offsets[s]]), int(self.hits.offsets[self.rec_offsets[s + 1]])
+        return a + np.flatnonzero(self.hit_chain[a:b] == np.uint32(k - int(self.offsets[s])))
+
+    def read_coords(self):
+        """Per-chain arrays in the ORIGINAL read's orientation: `read` (the read's index in the batch), `strand`, and qbeg /
+        qend -- for a strand-1 chain qbeg = L - qend, qend = L - qbeg of its reverse-complement coordinates."""
+        slot = self.chains["slot"].astype(np.int64)
+        q = self.chains["q"]
+        qb, qe = (q & 0xFFFF).astype(np.uint32), (q >> 16).astype(np.uint32)
+        if self.strands == 1:
+            return {"read": slot, "strand": np.zeros(len(slot), np.uint8), "qbeg": qb, "qend": qe}
+        strand = (slot & 1).astype(np.uint8)
+        L = np.asarray(self.lengths, np.uint32)[slot >> 1]
+        rev = strand == 1
+        return {"read": slot >> 1, "strand": strand, "qbeg": np.where(rev, L - qe, qb), "qend": np.where(rev, L - qb, qe)}
+
+    def best(self):
+        """Per read, the index of its heaviest chain over its slots, or -1 without chains; ties go to the lower slot, then to
+        the earlier chain."""
+        n_reads = (len(self.offsets) - 1) // self.strands
+        out = np.full(n_reads, -1, np.int64)
+        if len(self.chains):
+            read = self.chains["slot"].astype(np.int64) // self.strands
+            order = np.lexsort((np.arange(len(read)), -self.chains["weight"].astype(np.int64), read))
+            first = order[np.r_[True, read[order][1:] != read[order][:-1]]]
+            out[read[first]] = first
+        return out
+
+
 class Engine:
     """Owns the workspace for batches of up to `max_reads` reads of up to `max_len` bases.
 
@@ -992,6 +1045,18 @@ class Engine:
         _, n_rec = self.check_overflow()
         return _expand_hits(self.index, self.records, n_rec, max_occ, min_len, hit_cap)
 
+    def chain_seeds(self, max_occ=500, min_len=19, w=100, max_gap=10000):
+        """Chains of the batch this engine selected last (chain_seeds has the semantics): hits are located from the engine's
+        record buffer into device memory and chained there; only the results are copied back."""
+        r = getattr(self, "_reads_c", None)
+        if r is None:
+            raise ValueError("no batch has been selected yet")
+        _, n_rec = self.check_overflow()
+        n = int(r.n_reads)
+        rec_offsets = self.rec_off[: n + 1].cpu().numpy()
+        lengths = self.ds_len[:n].cpu().numpy().view(np.uint32)[0::2].copy() if self.strands == 2 else None
+        return _chain(self.index, self.records, n_rec, self.rec_off, rec_offsets, max_occ, min_len, w, max_gap, self.strands, lengths)
+
     def _grow(self):
         dev = self.device
         self.mem_cap = min(self.mem_cap * 4, (1 << 32) - 1)
@@ -1049,29 +1114,47 @@ def locate_hits(index: DeviceIndex, records, max_occ=500, min_len=0, hit_cap=Non
     require_cuda()
     recs = np.ascontiguousarray(records).view(RECORD_DTYPE).reshape(-1)
     n_rec = len(recs)
-    if n_rec and int((recs["sa_hi"][recs["sa_hi"] >= recs["sa_lo"]]).max(initial=0)) >= index.n_rows:
-        raise ValueError("a record's interval lies outside the index")
-    dev = torch.from_numpy(recs.view(np.uint8).reshape(-1)).to(index.device) if n_rec else torch.empty(16, dtype=torch.uint8, device=index.device)
+    _validate_records(index, recs)
+    dev =torch.from_numpy(recs.view(np.uint8).reshape(-1)).to(index.device) if n_rec else torch.empty(16, dtype=torch.uint8, device=index.device)
     return _expand_hits(index, dev, n_rec, max_occ, min_len, hit_cap)
 
 
-def _expand_hits(index, recs, n_rec, max_occ, min_len, hit_cap):
-    """gsm_hits_count + gsm_hits_locate over records already on the device (recs: uint8 tensor, n_rec x 16 bytes)."""
-    ssa = getattr(index, "ssa", None)
-    if index.sa is None and ssa is None:
+def _hit_params(index, max_occ, min_len):
+    if index.sa is None and getattr(index, "ssa", None) is None:
         raise ValueError("no suffix array on the device: call build_sampled_sa() before dropping it")
     max_occ, min_len = int(max_occ), int(min_len)
     if max_occ < 0 or min_len < 0:
         raise ValueError("max_occ and min_len must be >= 0")
+    return max_occ, min_len
+
+
+def _count_hits(index, recs, n_rec, max_occ, min_len):
+    """gsm_hits_count over records on the device -> hit_off (device int64, n_rec + 1 entries) and its host copy."""
+    dev = index.device
+    counts = torch.empty(max(n_rec, 1), dtype=torch.int32, device=dev)
+    off = torch.empty(n_rec + 1, dtype=torch.int64, device=dev)
+    tmp_bytes = C.c_uint64()
+    capi.check(capi.lib.gsm_hits_workspace_info(n_rec, C.byref(tmp_bytes)))
+    tmp = torch.empty(max(int(tmp_bytes.value), 8), dtype=torch.uint8, device=dev)
+    capi.check(capi.lib.gsm_hits_count(_ptr(recs), n_rec, max_occ, min_len, _ptr(counts), _ptr(off), _ptr(tmp), int(tmp_bytes.value), _stream()))
+    return off, off.cpu().numpy()
+
+
+def _locate_range(index, recs, off, a, b, max_occ, min_len, out, cap, status):
+    """gsm_hits_locate: the hits of records [a, b) to out (device, cap hits)."""
+    ssa = getattr(index, "ssa", None)
+    contigs = C.byref(index._contigs_c) if index.contigs is not None else None
+    ssa_p, sample = (_ptr(ssa), int(index.sa_sample)) if ssa is not None else (C.c_void_p(0), 0)
+    capi.check(capi.lib.gsm_hits_locate(C.byref(index.c), ssa_p, sample, contigs, _ptr(recs), _ptr(off), a, b, max_occ, min_len,
+                                        _ptr(out), cap, _ptr(status), _stream()))
+
+
+def _expand_hits(index, recs, n_rec, max_occ, min_len, hit_cap):
+    """gsm_hits_count + gsm_hits_locate over records already on the device (recs: uint8 tensor, n_rec x 16 bytes)."""
+    max_occ, min_len = _hit_params(index, max_occ, min_len)
     with torch.cuda.device(index.device):
         dev = index.device
-        counts = torch.empty(max(n_rec, 1), dtype=torch.int32, device=dev)
-        off = torch.empty(n_rec + 1, dtype=torch.int64, device=dev)
-        tmp_bytes = C.c_uint64()
-        capi.check(capi.lib.gsm_hits_workspace_info(n_rec, C.byref(tmp_bytes)))
-        tmp = torch.empty(max(int(tmp_bytes.value), 8), dtype=torch.uint8, device=dev)
-        capi.check(capi.lib.gsm_hits_count(_ptr(recs), n_rec, max_occ, min_len, _ptr(counts), _ptr(off), _ptr(tmp), int(tmp_bytes.value), _stream()))
-        offsets = off.cpu().numpy()
+        off, offsets = _count_hits(index, recs, n_rec, max_occ, min_len)
         total = int(offsets[-1])
         if total == 0:
             return HitResult(np.zeros(0, HIT_DTYPE), offsets)
@@ -1080,8 +1163,6 @@ def _expand_hits(index, recs, n_rec, max_occ, min_len, hit_cap):
         out = torch.empty(cap * 16, dtype=torch.uint8, device=dev)
         status = torch.zeros(1, dtype=torch.int64, device=dev)
         host = torch.empty(total * 16, dtype=torch.uint8, pin_memory=True)
-        contigs = C.byref(index._contigs_c) if index.contigs is not None else None
-        ssa_p, sample = (_ptr(ssa), int(index.sa_sample)) if ssa is not None else (C.c_void_p(0), 0)
         a = 0
         while a < n_rec:
             # records [a, b): as many as fit in cap hits (one at least)
@@ -1089,14 +1170,96 @@ def _expand_hits(index, recs, n_rec, max_occ, min_len, hit_cap):
             b = min(b, n_rec)
             h0, h1 = int(offsets[a]), int(offsets[b])
             if h1 > h0:
-                capi.check(capi.lib.gsm_hits_locate(C.byref(index.c), ssa_p, sample, contigs, _ptr(recs), _ptr(off), a, b, max_occ, min_len,
-                                                    _ptr(out), cap, _ptr(status), _stream()))
+                _locate_range(index, recs, off, a, b, max_occ, min_len, out, cap, status)
                 host[h0 * 16:h1 * 16].copy_(out[:(h1 - h0) * 16], non_blocking=True)
             a = b
         torch.cuda.current_stream().synchronize()
         if int(status.item()) != 0:
             raise capi.GsmError(capi.E_CAPACITY, "gsm_hits_locate: hit buffer overflow")
     return HitResult(host.numpy().view(HIT_DTYPE), offsets)
+
+
+def _device_hits(index, recs, n_rec, max_occ, min_len):
+    """Every hit of records on the device, left on the device: -> (hit_off device, its host copy, hits uint8 tensor of
+    total x 16 bytes, total)."""
+    off, offsets = _count_hits(index, recs, n_rec, max_occ, min_len)
+    total = int(offsets[-1])
+    hits = torch.empty(max(total, 1) * 16, dtype=torch.uint8, device=index.device)
+    if total:
+        status = torch.zeros(1, dtype=torch.int64, device=index.device)
+        _locate_range(index, recs, off, 0, n_rec, max_occ, min_len, hits, total, status)
+    return off, offsets, hits, total
+
+
+def _validate_records(index, recs):
+    if len(recs) and int((recs["sa_hi"][recs["sa_hi"] >= recs["sa_lo"]]).max(initial=0)) >= index.n_rows:
+        raise ValueError("a record's interval lies outside the index")
+
+
+def _chain_params(w, max_gap):
+    w, max_gap = int(w), int(max_gap)
+    if not (0 <= w < 1 << 32 and 0 <= max_gap < 1 << 32):
+        raise ValueError("w and max_gap must be in [0, 2^32)")
+    return w, max_gap
+
+
+def _chain(index, recs, n_rec, rec_off, rec_offsets, max_occ, min_len, w, max_gap, strands, lengths):
+    """Hits of the records on the device (never copied to the host in between), chained per slot (gsm_chain_seeds +
+    gsm_chains_collect); recs: uint8 tensor (n_rec x 16 bytes), rec_off: device int64 per slot, rec_offsets: its host copy."""
+    max_occ, min_len = _hit_params(index, max_occ, min_len)
+    w, max_gap = _chain_params(w, max_gap)
+    n_slots = len(rec_offsets) - 1
+    dev = index.device
+    with torch.cuda.device(dev):
+        off, offsets, hits, total = _device_hits(index, recs, n_rec, max_occ, min_len)
+        hit_chain = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
+        cnt = torch.empty(max(n_slots, 1), dtype=torch.int32, device=dev)
+        coff = torch.empty(n_slots + 1, dtype=torch.int64, device=dev)
+        need = C.c_uint64()
+        capi.check(capi.lib.gsm_chains_workspace_info(n_slots, total, C.byref(need)))
+        ws = torch.empty(max(int(need.value), 8), dtype=torch.uint8, device=dev)
+        capi.check(capi.lib.gsm_chain_seeds(_ptr(recs), _ptr(rec_off), n_slots, _ptr(hits), _ptr(off), total, w, max_gap, _ptr(hit_chain), _ptr(cnt),
+                                            _ptr(coff), _ptr(ws), int(need.value), _stream()))
+        chain_off = coff.cpu().numpy()
+        n_ch = int(chain_off[-1])
+        out = torch.empty(max(n_ch, 1) * 32, dtype=torch.uint8, device=dev)
+        status = torch.zeros(1, dtype=torch.int64, device=dev)
+        capi.check(capi.lib.gsm_chains_collect(_ptr(rec_off), n_slots, _ptr(off), total, _ptr(coff), _ptr(ws), int(need.value), _ptr(out), n_ch,
+                                               _ptr(status), _stream()))
+        h_chains = torch.empty(n_ch * 32, dtype=torch.uint8, pin_memory=True)
+        h_hits = torch.empty(total * 16, dtype=torch.uint8, pin_memory=True)
+        h_ids = torch.empty(total, dtype=torch.int32, pin_memory=True)
+        h_chains.copy_(out[:n_ch * 32], non_blocking=True)
+        h_hits.copy_(hits[:total * 16], non_blocking=True)
+        h_ids.copy_(hit_chain[:total], non_blocking=True)
+        torch.cuda.current_stream().synchronize()
+        if int(status.item()) != 0:
+            raise capi.GsmError(capi.E_CAPACITY, "gsm_chains_collect: chain buffer overflow")
+    hr = HitResult(h_hits.numpy().view(HIT_DTYPE), offsets)
+    return ChainResult(h_chains.numpy().view(CHAIN_DTYPE), chain_off, hr, h_ids.numpy().view(np.uint32), rec_offsets, strands, lengths)
+
+
+def chain_seeds(index: DeviceIndex, result, max_occ=500, min_len=19, w=100, max_gap=10000):
+    """BWA-MEM's seed chaining (mem_chain) of every slot of an SmemResult (Engine.run, PipelinedEngine.run*): its records
+    are expanded into hits on the device (locate_hits with max_occ / min_len, BWA's -c and -k), and each slot's hits -- in
+    record order, then suffix-array row order -- are grouped into co-linear chains on one sequence (test_and_merge with band
+    w and max_gap, BWA's -w and max_chain_gap; hits that span two sequences are skipped).  A slot's chains are ordered by
+    (contig, rbeg of the first seed), ties in creation order; `lower` among tied chains is the one created first.  Only the
+    chains, the hits and their chain ids come back to the host -> ChainResult."""
+    require_cuda()
+    recs = np.ascontiguousarray(result.records).view(RECORD_DTYPE).reshape(-1)
+    _validate_records(index, recs)
+    rec_offsets = np.ascontiguousarray(result.offsets, np.int64)
+    if len(rec_offsets) < 1 or rec_offsets[0] != 0 or rec_offsets[-1] != len(recs) or (np.diff(rec_offsets) < 0).any():
+        raise ValueError("result.offsets must rise from 0 to the number of records")
+    if result.strands == 2 and result.lengths is None:
+        raise ValueError("a strands=2 result needs its read lengths")
+    n_rec = len(recs)
+    with torch.cuda.device(index.device):
+        dev = torch.from_numpy(recs.view(np.uint8).reshape(-1)).to(index.device) if n_rec else torch.empty(16, dtype=torch.uint8, device=index.device)
+        rec_off = torch.from_numpy(rec_offsets).to(index.device)
+        return _chain(index, dev, n_rec, rec_off, rec_offsets, max_occ, min_len, w, max_gap, result.strands,
+                      None if result.lengths is None else np.asarray(result.lengths, np.uint32).copy())
 
 
 def set_rmi_prefilter(on=True):

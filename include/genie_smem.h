@@ -480,6 +480,54 @@ int gsm_hits_locate(const gsm_dev_index* idx, const uint32_t* ssa, uint32_t samp
                     const gsm_record* recs, const uint64_t* hit_off, uint64_t rec_begin, uint64_t rec_end, uint32_t max_occ,
                     uint32_t min_len, gsm_hit* out, uint64_t out_cap, uint64_t* status8, void* stream);
 
+/* ------------------------------------------------------------------ chains: located hits -> co-linear seed chains
+ * BWA-MEM's mem_chain (test_and_merge, mem_chain_weight) per SLOT: slot s = read s of the batch, or with a strand-doubled
+ * batch read s >> 1 on strand s & 1.  The records of slot s are recs[rec_off[s] .. rec_off[s+1]) (the engine's rec_off),
+ * the hits of record r are hits[hit_off[r] .. hit_off[r+1]) (gsm_hits_count / gsm_hits_locate).  The slot's seeds are its
+ * hits in record order, then hit order; the seed of hit h of record r is qbeg = r.qstart, len = r.qend - r.qstart,
+ * rbeg = h.offset on sequence h.contig.  A hit flagged GSM_HIT_SPANS is skipped (BWA's rid < 0).
+ *
+ * The slot's chains are ordered by (contig, pos), pos = rbeg of the first seed; each seed is tested against `lower`, the
+ * chain with the largest key <= (contig, rbeg) -- the one created first when several share it -- by BWA's test_and_merge
+ * with 64-bit signed differences: contained (qbeg >= first.qbeg, qbeg + len <= last.qbeg + last.len, and the same on the
+ * reference) -> not appended; appended if y = rbeg - last.rbeg >= 0, |x - y| <= w (x = qbeg - last.qbeg),
+ * x - last.len < max_gap and y - last.len < max_gap; otherwise, or without `lower`, the seed starts a new chain.  BWA's
+ * defaults: w = 100 (-w), max_gap = 10000 (max_chain_gap).
+ *
+ * Output: the chains of every slot in slot order, within a slot in (contig, pos) order with ties in creation order; a chain's
+ * id is its index within its slot in that order.  hit_chain[h] = id of the chain hit h was appended to, GSM_CHAIN_CONTAINED |
+ * id when contained, GSM_CHAIN_NONE for a spanning hit. */
+#define GSM_CHAIN_NONE 0xFFFFFFFFu
+#define GSM_CHAIN_CONTAINED 0x80000000u
+
+typedef struct {
+    uint32_t slot;     /* slot in the batch (not the read id) */
+    uint32_t contig;
+    uint32_t rbeg;     /* rbeg of the first seed */
+    uint32_t rend;     /* max rbeg + len over the member seeds */
+    uint32_t q;        /* qbeg | qend << 16: min qbeg, max qend over the members; reverse-complement coordinates on a strand-1 slot */
+    uint32_t weight;   /* mem_chain_weight: min(non-overlapping query coverage, non-overlapping reference coverage) */
+    uint32_t n_seeds;  /* member seeds (contained seeds are not members) */
+    uint32_t reserved; /* 0 */
+} gsm_chain;
+
+/* Bytes of device workspace for n_slots slots over a hits array of n_hits entries (host arithmetic, no device needed):
+ * 84 bytes per hit (a slot's scratch sits at its first hit) plus a few bytes per slot. */
+int gsm_chains_workspace_info(uint64_t n_slots, uint64_t n_hits, uint64_t* bytes);
+
+/* Phase 1: chain every slot.  hit_chain (n_hits u32) receives the ids, chain_cnt (n_slots u32) the chains per slot and
+ * chain_off (n_slots + 1 u64) their exclusive scan, chain_off[n_slots] = the total.  All pointers are device memory; the
+ * workspace is the caller's (gsm_chains_workspace_info) and must be passed unchanged to phase 2.  GSM_E_CAPACITY for a
+ * short workspace.  Asynchronous on stream. */
+int gsm_chain_seeds(const gsm_record* recs, const uint64_t* rec_off, uint64_t n_slots, const gsm_hit* hits, const uint64_t* hit_off,
+                    uint64_t n_hits, uint32_t w, uint32_t max_gap, uint32_t* hit_chain, uint32_t* chain_cnt, uint64_t* chain_off,
+                    void* workspace, uint64_t workspace_bytes, void* stream);
+
+/* Phase 2: chain k of the batch to out[k] (device, out_cap entries).  Nothing is written at or past out_cap; if the batch
+ * holds more chains, bit 0 of *status8 (device uint64) is set.  Asynchronous on stream. */
+int gsm_chains_collect(const uint64_t* rec_off, uint64_t n_slots, const uint64_t* hit_off, uint64_t n_hits, const uint64_t* chain_off,
+                       const void* workspace, uint64_t workspace_bytes, gsm_chain* out, uint64_t out_cap, uint64_t* status8, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
