@@ -7,7 +7,7 @@
 //     dynamic read queue), bidirectional FM extension enumerating every maximal exact match of the read; per iteration
 //     every lane runs its control and the warp executes ONE uniform memory section (seed-table entry / bucket / suffix-array
 //     value / text words).  Finished reads hand their match lists over cooperatively (flush_finished): ordered, field by
-//     field, and with the BWA-SMEM picks already made.  k_sweep (lane pairs, round 1) is kept behind GSM_SWEEP_LPR=2.
+//     field, and with the BWA-SMEM picks already made.
 //   * BWA-SMEM selection: k_select_bwa_picked (count + min_len filter where the sweep made the picks), k_select<BWA> (one
 //     thread per read, Selector::run_bwa) for the reads it queues, k_select_bwa_finish.  LUT-SMEM takes the same records
 //     (get_smems_lut == get_SMEMS with min_len 1 on reads of >= K bases, DESIGN.md section 3) unless the frame machine is
@@ -54,9 +54,8 @@ static int g_lut_frame_machine = getenv("GSM_LUT_MACHINE") ? atoi(getenv("GSM_LU
 static int g_rmi_prefilter = getenv("GSM_RMI_PREFILTER") ? atoi(getenv("GSM_RMI_PREFILTER")) : 1;
 constexpr uint8_t READ_PENDING = 0xFFu;      // read_status while a pre-filtered RMI batch waits for the frame machine (never survives a select)
 constexpr int SELECT_THREADS = 128;
-constexpr int SELECT_BLOCKS = 7;             // k_select_seeded: resident blocks per SM the registers are allocated for
-constexpr int SELECT_DEFAULT_OPT_LUT = 1;    // measured per method (tools/sweep_ab.py, profiles/r02_notes.md)
-constexpr int SELECT_DEFAULT_OPT_RMI = 3;
+constexpr int SELECT_BLOCKS = 7;             // k_select_seeded: resident blocks per SM the registers are allocated for (72 registers;
+                                             // 6 and 8 measured slower for both methods)
 constexpr uint32_t SELECT_STAGE = 64;   // staged records per selection thread; reads emitting more are run twice (see DevSelCtx::close)
 
 // ===================================================================================== select
@@ -496,10 +495,8 @@ __device__ __noinline__ LiteralOut literal_lookups(const SelectArgs& a, const ui
 // ARITH (RMI only): 1 = the launch has a usable seed table (seed_K <= K) and the None rows, so every lookup is the probe-free
 // rmi_arith_lookup and the probe-based phases are compiled out (fewer registers for the path that always runs);
 // 2 = as 1, the k-mer's true bounds read from the dense table of gsm_rmi_bounds_build (one fetch, no backward steps).
-// MB: resident blocks per SM the register allocation aims at (7: 72 registers; 8: 64 with spills and 6: 80 measured slower)
-// OPT: bit 0 = two (thread, window) pairs per lane and trip of pass 1, bit 1 = prefetch of the thread's next read
-template <int METHOD, int ARITH = 0, int MB = 8, int OPT = 0>
-__global__ void __launch_bounds__(SELECT_THREADS, MB) k_select_seeded(const __grid_constant__ SelectArgs a) {
+template <int METHOD, int ARITH>
+__global__ void __launch_bounds__(SELECT_THREADS, SELECT_BLOCKS) k_select_seeded(const __grid_constant__ SelectArgs a) {
     using CtxT = DevSelCtx<METHOD>;
     using Sel = Selector<CtxT>;
     const size_t gtid = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -517,8 +514,10 @@ __global__ void __launch_bounds__(SELECT_THREADS, MB) k_select_seeded(const __gr
     uint16_t* const items = reinterpret_cast<uint16_t*>(sel_smem + 2u * a.K * WIN_STRIDE + WIN_MASKS * SELECT_THREADS)
                             + (threadIdx.x >> 5) * (a.K * 32u);                                // this warp's (lane, window) pairs of a round
     const uint32_t lane = threadIdx.x & 31u;
-    constexpr int IPL = (OPT & 1) ? 2 : 1;                 // (thread, window) pairs per lane and trip of pass 1
-    constexpr bool PREFETCH = (OPT & 2) != 0;              // the thread's next read is brought into the L2 while this one runs
+    // measured per method (tools/sweep_ab.py, profiles/r02_notes.md): two (thread, window) pairs per lane and trip of pass 1,
+    // and for the probe-free RMI lookups the thread's next read brought into the L2 while this one runs
+    constexpr int IPL = 2;
+    constexpr bool PREFETCH = METHOD == GSM_METHOD_RMI && ARITH != 0;
     uint32_t nx_chunk = 0, nx_off = 0;                     // PREFETCH: where the next read's bases and match list are
 
     auto close_read = [&](uint8_t status) {
@@ -1160,64 +1159,39 @@ int device_ready() {
     return GSM_OK;
 }
 
-// Which sweep kernel runs a batch: lane pairs (k_sweep) or one lane per read with the read in shared memory
-// (k_sweep1<false>) for reads up to SWEEP1_SMEM_MAX_LEN bases -- GSM_SWEEP_LPR=1|2 picks between them -- and
-// k_sweep1<true> (bases from global memory, grid sized by the staging budget) for anything longer, up to 65535 bases.
-enum SweepKind { SWEEP_PAIR = 0, SWEEP_LANE = 1, SWEEP_LANE_LONG = 2 };
-
-int sweep_kind(uint32_t max_len) {
-    static const int lpr = getenv("GSM_SWEEP_LPR") ? atoi(getenv("GSM_SWEEP_LPR")) : 1;
-    if (max_len > SWEEP1_SMEM_MAX_LEN) return SWEEP_LANE_LONG;
-    return lpr == 2 ? SWEEP_PAIR : SWEEP_LANE;
-}
-
-int sweep_blocks_env() {       // GSM_SWEEP_BLOCKS=6|8: the lane kernel compiled for more resident blocks (fewer registers); A/B switch
-    static const int v = getenv("GSM_SWEEP_BLOCKS") ? atoi(getenv("GSM_SWEEP_BLOCKS")) : 0;
-    return v;
+// Which sweep kernel runs a batch: k_sweep1<false> with the read in shared memory for reads up to SWEEP1_SMEM_MAX_LEN
+// bases, k_sweep1<true> (bases from global memory, grid sized by the staging budget) for anything longer, up to 65535
+// bases; UNIQ when the suffix array and the packed text are on the device (the unique-match shortcut).
+using SweepKernel = void (*)(const SweepArgs);
+bool sweep_long(uint32_t max_len) { return max_len > SWEEP1_SMEM_MAX_LEN; }
+SweepKernel sweep_kernel(bool long_reads, bool uniq) {
+    if (long_reads) return uniq ? k_sweep1<true, true> : k_sweep1<true, false>;
+    return uniq ? k_sweep1<false, true> : k_sweep1<false, false>;
 }
 
 int sweep_grid(uint32_t max_len, int* blocks) {
-    int dev = 0, sms = 0, per_sm = 0;
+    int dev = 0, sms = 0;
     GSM_CUDA(cudaGetDevice(&dev));
     GSM_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    const int kind = sweep_kind(max_len);
-    if (kind == SWEEP_LANE) {
-        const size_t smem = sweep1_smem_bytes(max_len, false);
-        GSM_CUDA(cudaFuncSetAttribute(k_sweep1<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        GSM_CUDA(cudaFuncSetAttribute(k_sweep1<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        GSM_CUDA(cudaFuncSetAttribute(k_sweep1<false, true, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        GSM_CUDA(cudaFuncSetAttribute(k_sweep1<false, true, SWEEP1_MIN_BLOCKS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        GSM_CUDA(cudaFuncSetAttribute(k_sweep1<false, true, SWEEP1_MIN_BLOCKS, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        GSM_CUDA(cudaFuncSetAttribute(k_sweep1<false, true, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        int a0 = 0, a1 = 0;                 // the grid must be resident for either instantiation (with / without the text shortcut)
-        GSM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a0, k_sweep1<false, false>, SWEEP1_THREADS, smem));
-        GSM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a1, k_sweep1<false, true>, SWEEP1_THREADS, smem));
-        per_sm = a0 < a1 ? a0 : a1;
-        if (sweep_blocks_env() == 6) GSM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sweep1<false, true, 6>, SWEEP1_THREADS, smem));
-        if (sweep_blocks_env() == 8) GSM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sweep1<false, true, 8>, SWEEP1_THREADS, smem));
-    } else if (kind == SWEEP_LANE_LONG) {
-        int a0 = 0, a1 = 0;
-        GSM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a0, k_sweep1<true, false>, SWEEP1_THREADS, sweep1_smem_bytes(max_len, true)));
-        GSM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a1, k_sweep1<true, true>, SWEEP1_THREADS, sweep1_smem_bytes(max_len, true)));
-        per_sm = a0 < a1 ? a0 : a1;
-    } else {
-        const size_t smem = sweep_smem_bytes(max_len);
-        GSM_CUDA(cudaFuncSetAttribute(k_sweep, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        GSM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sweep, SWEEP_THREADS, smem));
+    const bool long_reads = sweep_long(max_len);
+    const size_t smem = sweep1_smem_bytes(max_len, long_reads);
+    int a[2] = {0, 0};                  // the grid must be resident for either instantiation (with / without the text shortcut)
+    for (int uniq = 0; uniq < 2; ++uniq) {
+        const SweepKernel k = sweep_kernel(long_reads, uniq != 0);
+        GSM_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        GSM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a[uniq], k, SWEEP1_THREADS, smem));
     }
+    const int per_sm = a[0] < a[1] ? a[0] : a[1];
     if (per_sm < 1) return fail(GSM_E_CAPACITY, "read length too large for the sweep kernel's shared memory");
     *blocks = sms * per_sm;
-    if (kind == SWEEP_LANE_LONG) {        // long reads: as many blocks as the staging budget allows (2 x max_len x 16 B per lane)
+    if (long_reads) {                   // long reads: as many blocks as the staging budget allows (2 x max_len x 16 B per lane)
         const uint64_t fit = SWEEP1_LONG_SCRATCH / ((uint64_t)SWEEP1_THREADS * 2ull * max_len * 16ull);
         if ((uint64_t)*blocks > fit) *blocks = fit < 1 ? 1 : (int)fit;
     }
     return GSM_OK;
 }
 
-uint64_t sweep_scratch_bytes(int blocks, uint32_t max_len) {
-    const uint64_t reads_per_block = sweep_kind(max_len) == SWEEP_PAIR ? SWEEP_GROUPS : SWEEP1_THREADS;
-    return (uint64_t)blocks * reads_per_block * 2ull * max_len * 16ull;
-}
+uint64_t sweep_scratch_bytes(int blocks, uint32_t max_len) { return (uint64_t)blocks * SWEEP1_THREADS * 2ull * max_len * 16ull; }
 
 uint32_t select_stage_stride(uint32_t max_len) { return max_len < SELECT_STAGE ? max_len : SELECT_STAGE; }
 
@@ -1241,27 +1215,14 @@ int resident_grid(Kern kern, int threads, size_t smem, int cap, int* blocks) {
     return GSM_OK;
 }
 
-template <int METHOD, int ARITH, int MB, int OPT>
-int launch_seeded1(const SelectArgs& se, int cap, cudaStream_t stream) {
-    int grid = cap;
-    const size_t smem = select_smem_bytes(se.K);                          // at most 44 KB (K <= 32)
-    const int st = resident_grid(k_select_seeded<METHOD, ARITH, MB, OPT>, SELECT_THREADS, smem, cap, &grid);
-    if (st) return st;
-    k_select_seeded<METHOD, ARITH, MB, OPT><<<grid, SELECT_THREADS, smem, stream>>>(se);
-    return GSM_OK;
-}
-// A/B switch (tools/sweep_ab.py): GSM_SELECT_OPT bit 0 = two (thread, window) pairs per lane and trip of pass 1, bit 1 = prefetch
-// of the thread's next read.  Resident blocks per SM: 7 (72 registers; 6 and 8 measured slower for both methods).
 template <int METHOD, int ARITH>
 int launch_seeded(const SelectArgs& se, int cap, cudaStream_t stream) {
-    static const int opt = getenv("GSM_SELECT_OPT") ? atoi(getenv("GSM_SELECT_OPT")) : (METHOD == GSM_METHOD_LUT ? SELECT_DEFAULT_OPT_LUT : SELECT_DEFAULT_OPT_RMI);
-    switch (opt) {
-        case 0: return launch_seeded1<METHOD, ARITH, SELECT_BLOCKS, 0>(se, cap, stream);
-        case 1: return launch_seeded1<METHOD, ARITH, SELECT_BLOCKS, 1>(se, cap, stream);
-        case 2: return launch_seeded1<METHOD, ARITH, SELECT_BLOCKS, 2>(se, cap, stream);
-        case 3: return launch_seeded1<METHOD, ARITH, SELECT_BLOCKS, 3>(se, cap, stream);
-    }
-    return fail(GSM_E_INVALID, "GSM_SELECT_OPT must be 0..3");
+    int grid = cap;
+    const size_t smem = select_smem_bytes(se.K);                          // at most 44 KB (K <= 32)
+    const int st = resident_grid(k_select_seeded<METHOD, ARITH>, SELECT_THREADS, smem, cap, &grid);
+    if (st) return st;
+    k_select_seeded<METHOD, ARITH><<<grid, SELECT_THREADS, smem, stream>>>(se);
+    return GSM_OK;
 }
 
 }  // namespace
@@ -1298,7 +1259,7 @@ int gsm_smem_workspace_info(uint64_t n_reads, uint32_t max_len, gsm_workspace_in
     out->quad_scratch_bytes = sweep_bytes > sel_bytes ? sweep_bytes : sel_bytes;
     out->scan_tmp_bytes = ((n_reads + SCAN_TILE - 1) / SCAN_TILE + 2) * 8ull;
     out->grid_blocks = (uint32_t)sb;
-    out->block_threads = sweep_kind(max_len) == SWEEP_PAIR ? SWEEP_THREADS : SWEEP1_THREADS;
+    out->block_threads = SWEEP1_THREADS;
     return GSM_OK;
 }
 
@@ -1540,31 +1501,14 @@ int gsm_smem_sweep(const gsm_dev_index* ix, const gsm_dev_reads* rd, gsm_workspa
     SweepArgs sa;
     sa.fwd = (const uint4*)ix->fwd_buckets; sa.rev = (const uint4*)ix->rev_buckets; sa.meta = make_meta(ix);
     sa.reads = (const uint4*)rd->packed; sa.chunk_off = rd->chunk_off; sa.len = rd->len; sa.n_reads = (uint32_t)rd->n_reads;
-    sa.read_u4 = sweep_read_u4(rd->max_len); sa.pack_u4 = sweep_pack_u4(rd->max_len); sa.max_len = rd->max_len;
+    sa.max_len = rd->max_len;
     sa.seed_tab = (const uint4*)ix->seed_table; sa.seed_K = ix->seed_table ? ix->seed_K : 0u;
     if (sa.seed_tab && (sa.seed_K < 1 || sa.seed_K > 16)) return fail(GSM_E_INVALID, "seed table K must be in 1..16");
     sa.mem_pool = (uint4*)ws->mem_pool; sa.mem_cap = ws->mem_cap; sa.mem_off = ws->mem_off; sa.mem_cnt = ws->mem_cnt;
     sa.scratch = (uint4*)ws->quad_scratch; sa.counters = (unsigned long long*)ws->counters;
-    // unique-match shortcut of the lane kernels: needs the suffix array and the packed text on the device (GSM_SWEEP_UNIQ=0 disables)
-    static const int uniq_env = getenv("GSM_SWEEP_UNIQ") ? atoi(getenv("GSM_SWEEP_UNIQ")) : 1;
     sa.sa = ix->sa; sa.text = ix->text2bit; sa.n_bases = (uint32_t)(ix->n_rows - 1);
-    const bool uniq = uniq_env != 0 && ix->sa && ix->text2bit;
-    const int kind = sweep_kind(rd->max_len);
-    if (kind == SWEEP_LANE) {
-        static const int stats = getenv("GSM_SWEEP_STATS") ? atoi(getenv("GSM_SWEEP_STATS")) : 0;
-        static const int paired = getenv("GSM_SWEEP_PAIRED") ? atoi(getenv("GSM_SWEEP_PAIRED")) : 0;      // A/B: buckets as one 64-byte request per lane pair
-        if (uniq && paired) { k_sweep1<false, true, SWEEP1_MIN_BLOCKS, false, true><<<sb, SWEEP1_THREADS, sweep1_smem_bytes(rd->max_len, false), stream>>>(sa); GSM_CUDA(cudaGetLastError()); return GSM_OK; }
-        if (uniq && stats) k_sweep1<false, true, SWEEP1_MIN_BLOCKS, true><<<sb, SWEEP1_THREADS, sweep1_smem_bytes(rd->max_len, false), stream>>>(sa);
-        else if (uniq && sweep_blocks_env() == 6) k_sweep1<false, true, 6><<<sb, SWEEP1_THREADS, sweep1_smem_bytes(rd->max_len, false), stream>>>(sa);
-        else if (uniq && sweep_blocks_env() == 8) k_sweep1<false, true, 8><<<sb, SWEEP1_THREADS, sweep1_smem_bytes(rd->max_len, false), stream>>>(sa);
-        else if (uniq) k_sweep1<false, true><<<sb, SWEEP1_THREADS, sweep1_smem_bytes(rd->max_len, false), stream>>>(sa);
-        else k_sweep1<false, false><<<sb, SWEEP1_THREADS, sweep1_smem_bytes(rd->max_len, false), stream>>>(sa);
-    } else if (kind == SWEEP_LANE_LONG) {
-        if (uniq) k_sweep1<true, true><<<sb, SWEEP1_THREADS, sweep1_smem_bytes(rd->max_len, true), stream>>>(sa);
-        else k_sweep1<true, false><<<sb, SWEEP1_THREADS, sweep1_smem_bytes(rd->max_len, true), stream>>>(sa);
-    } else {
-        k_sweep<<<sb, SWEEP_THREADS, sweep_smem_bytes(rd->max_len), stream>>>(sa);
-    }
+    const bool long_reads = sweep_long(rd->max_len);
+    sweep_kernel(long_reads, ix->sa && ix->text2bit)<<<sb, SWEEP1_THREADS, sweep1_smem_bytes(rd->max_len, long_reads), stream>>>(sa);
     GSM_CUDA(cudaGetLastError());
     return GSM_OK;
 }
@@ -1631,8 +1575,7 @@ int gsm_smem_select(int method, const gsm_dev_index* ix, const gsm_dev_reads* rd
         // reads whose picks the sweep made need no pass over their lists; the others queue up (4 read numbers per 16-byte
         // slot of the record pool's last eighth) for the one-thread-per-read kernel
         const uint64_t reserve = ws->rec_cap / 8;
-        static const bool use_picks = !(getenv("GSM_BWA_PICKS") && atoi(getenv("GSM_BWA_PICKS")) == 0);
-        if (use_picks && reserve * 4 >= rd->n_reads) {
+        if (reserve * 4 >= rd->n_reads) {
             se.rec_cap = ws->rec_cap - reserve;
             uint32_t* queue = (uint32_t*)((uint4*)ws->rec_tmp + se.rec_cap);
             GSM_CUDA(cudaMemsetAsync((unsigned long long*)ws->counters + 4, 0, 3 * sizeof(uint64_t), stream));    // queue length, mode, records
@@ -1668,7 +1611,7 @@ int gsm_smem_select(int method, const gsm_dev_index* ix, const gsm_dev_reads* rd
         if (method == GSM_METHOD_LUT) st = launch_seeded<GSM_METHOD_LUT, 0>(se, lb, stream);
         else if (se.rmi_bounds) st = launch_seeded<GSM_METHOD_RMI, 2>(se, lb, stream);
         else if (arith) st = launch_seeded<GSM_METHOD_RMI, 1>(se, lb, stream);
-        else st = launch_seeded1<GSM_METHOD_RMI, 0, SELECT_BLOCKS, 0>(se, lb, stream);
+        else st = launch_seeded<GSM_METHOD_RMI, 0>(se, lb, stream);
         if (st) return st;
         int dev = 0, sms = 148;
         GSM_CUDA(cudaGetDevice(&dev));

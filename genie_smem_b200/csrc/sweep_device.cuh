@@ -1,26 +1,19 @@
-// Device side of the sweep kernels.
-//   k_sweep1 (default): ONE LANE PER READ, 32 reads in flight per warp.  Every iteration each lane runs its per-read control
+// Device side of the sweep kernel.
+//   k_sweep1: ONE LANE PER READ, 32 reads in flight per warp.  Every iteration each lane runs its per-read control
 //   (sweep_logic.cuh: registers and shared memory only) and then the whole warp executes ONE uniform memory section -- a
 //   predicated seed-table fetch, a predicated suffix-array / text fetch, and the two 256-bit loads of one rank bucket with
 //   the bit-plane masks built once and popcounted below both offsets (lane_step) -- so all 32 chains' fetches are in flight
 //   together.  Finished reads hand their matches to the pool cooperatively (flush_finished): one atomic per warp,
 //   coalesced copies, lists of up to 64 matches ordered and stored field by field, the BWA-SMEM picks of lists of up to 32
 //   made on the way.
-//   k_sweep (GSM_SWEEP_LPR=2, round 1): two lanes ("a pair") per read, one bucket half each, halves summed with one shuffle
-//   (pair_step); 16 reads per warp.  (A 4-lane variant with 128-bit loads was measured first: 78 M reads/s against 103 M for
-//   pairs, 187 M for one lane per read on the same bench -- profiles/r01_notes.md, r02_notes.md.)
+//   One lane per read measured fastest: 187 M reads/s against 103 M for two lanes per read (one bucket half each) and
+//   78 M for four lanes with 128-bit loads on the same bench (profiles/r01_notes.md, r02_notes.md).
 #pragma once
 #include <cuda_runtime.h>
 
 #include "sweep_logic.cuh"
 
 namespace gsm {
-
-constexpr int SWEEP_THREADS = 128;
-constexpr int SWEEP_LPR = 2;                              // lanes per read
-constexpr int SWEEP_GROUPS = SWEEP_THREADS / SWEEP_LPR;   // reads in flight per block
-constexpr int SWEEP_CAP = 12;                             // candidates kept in shared memory per read
-constexpr int SWEEP_MIN_BLOCKS = 8;
 
 // mem_cnt[read]: number of maximal matches in the low 30 bits, and how the sweep left the list
 constexpr uint32_t MEMS_ORDERED = 0x80000000u;   // ascending and field by field (n start|end words, n lo, n count, n sweep ordinals)
@@ -35,8 +28,6 @@ struct SweepArgs {
     const uint32_t* chunk_off;
     const uint32_t* len;
     uint32_t n_reads;
-    uint32_t read_u4;        // uint4 slots of shared memory per read for its unpacked bases
-    uint32_t pack_u4;        // uint4 slots per read for its packed words (k-mer codes of the seed table)
     uint32_t max_len;
     const uint4* seed_tab;   // optional 4^seed_K x {fwd lo, count, rev lo, 0} (gsm_seed_table_build), else NULL
     uint32_t seed_K;
@@ -44,16 +35,15 @@ struct SweepArgs {
     unsigned long long mem_cap;
     uint32_t* mem_off;
     uint32_t* mem_cnt;
-    uint4* scratch;          // per pair: [0, max_len) match staging, [max_len, 2 max_len) candidate spill
+    uint4* scratch;          // per lane: [0, max_len) match staging, [max_len, 2 max_len) candidate spill
     unsigned long long* counters;
-    const uint32_t* sa;      // unique-match shortcut of the lane kernels (k_sweep1<.., true>): suffix array (1-based values) ...
+    const uint32_t* sa;      // unique-match shortcut (k_sweep1<.., true>): suffix array (1-based values) ...
     const uint32_t* text;    // ... and the 2-bit packed text (MSB-first, readable 2 words past its end)
     uint32_t n_bases;
 };
 
-// Shared memory: [per pair: SWEEP_CAP candidates of 16 B {end, lo, cnt, -}, then
-// the read's bases one per byte, then its packed words][16 B pad].  Indexed through one extern array so that
-// the compiler emits LDS/STS.
+// Shared memory: [per lane: SWEEP1_CAP candidates of 16 B {end, lo, cnt, -}, then (short reads) the read's packed
+// words][16 B pad] (sweep1_lane_u4).  Indexed through one extern array so that the compiler emits LDS/STS.
 extern __shared__ uint4 g_sweep_smem[];
 
 // one 32-byte half of a bucket: a single 256-bit read-only load
@@ -65,8 +55,9 @@ __device__ __forceinline__ Half ldg_half(const uint4* halves_base, size_t half_i
     return h;
 }
 
-// One FM extension step executed by all pairs of a warp together.  Every lane passes its pair's
-// operands; `active` pairs get their result, inactive ones issue no loads.  g = lane within pair.
+// One FM extension step by a lane pair (k_backsearch, k_add_one), all pairs of the warp together: each lane of a pair
+// loads one half of the bucket and the halves' counts are summed with shuffles.  Every lane passes its pair's operands;
+// `active` pairs get their result, inactive ones issue no loads.  g = lane within pair.
 __device__ __forceinline__ StepOut pair_step(const uint4* __restrict__ bk, uint32_t P0, uint32_t P1, uint32_t ch, uint32_t Cc,
                                              uint32_t primary, uint32_t g, bool active) {
     constexpr uint32_t FULLM = 0xFFFFFFFFu;
@@ -100,117 +91,10 @@ __device__ __forceinline__ uint4 ldg_seed(const uint4* p) {
     return v;
 }
 
-// byte of four 2-bit bases (MSB first) -> four bytes, first base at the lowest address (no table: one multiply)
-__device__ __forceinline__ uint32_t spread4(uint32_t x) { return ((x * 0x01004010u) | (x >> 6)) & 0x03030303u; }
-
-struct DevSweepCtx {
-    const SweepArgs& a;
-    uint32_t cand0;       // index (uint4) of this pair's candidate slots
-    uint32_t bytes0;      // byte offset of this pair's unpacked read
-    uint32_t words0;      // word offset of this pair's packed read
-    uint4* stage;         // global: match staging of this pair
-    uint4* spill;         // global: candidate spill of this pair
-    uint32_t g, gmask, gbase;
-
-    __device__ __forceinline__ bool fetch(uint32_t& rid, uint32_t& L) {
-        unsigned long long r = 0;
-        if (g == 0) r = atomicAdd(&a.counters[3], 1ull);
-        r = __shfl_sync(gmask, r, gbase);
-        if (r >= a.n_reads) return false;
-        rid = (uint32_t)r;
-        L = __ldg(a.len + rid);
-        const uint32_t off = __ldg(a.chunk_off + rid);
-        const uint32_t nch = (L + 63u) >> 6;
-        uint4* dst = g_sweep_smem + (bytes0 >> 4);
-        __syncwarp(gmask);                       // both lanes are done with the previous read's bases
-        for (uint32_t c = g; c < nch; c += SWEEP_LPR) {
-            const uint4 v = __ldg(a.reads + (size_t)off + c);
-            g_sweep_smem[(words0 >> 2) + c] = v;
-            const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-            for (int k = 0; k < 4; ++k)          // 16 packed bases -> 16 bytes, first base at the lowest address
-                if (c * 4 + k < a.read_u4)
-                    dst[c * 4 + k] = make_uint4(spread4(w[k] >> 24), spread4((w[k] >> 16) & 0xFFu), spread4((w[k] >> 8) & 0xFFu), spread4(w[k] & 0xFFu));
-        }
-        __syncwarp(gmask);
-        return true;
-    }
-    __device__ __forceinline__ uint32_t base(uint32_t pos) const {
-        return reinterpret_cast<const uint8_t*>(g_sweep_smem)[bytes0 + pos];
-    }
-    __device__ __forceinline__ uint32_t seed_k() const { return a.seed_K; }
-    // the unique-match shortcut of sweep_logic.cuh stays compiled out of the kernel: measured slower (profiles/r01_notes.md)
-    __device__ __forceinline__ constexpr bool uniq() const { return false; }
-    __device__ __forceinline__ constexpr bool uniq_back() const { return false; }
-    // code of q[pos:pos+K): top 2K bits of the 64-bit window starting at base pos (MSB-first packing)
-    __device__ __forceinline__ uint32_t kmer(uint32_t pos) const {
-        const uint32_t* w = reinterpret_cast<const uint32_t*>(g_sweep_smem) + words0 + (pos >> 4);
-        return __funnelshift_l(w[1], w[0], 2u * (pos & 15u)) >> (32u - 2u * a.seed_K);
-    }
-    __device__ __forceinline__ void cand_put(uint32_t i, uint32_t j, uint32_t lo, uint32_t cnt) {
-        if (i < (uint32_t)SWEEP_CAP) g_sweep_smem[cand0 + i] = make_uint4(j, lo, cnt, 0u);   // same value from both lanes
-        else if (g == 0) __stcg(spill + (i - SWEEP_CAP), make_uint4(j, lo, cnt, 0u));
-    }
-    __device__ __forceinline__ void cand_get(uint32_t i, uint32_t& j, uint32_t& lo, uint32_t& cnt) const {
-        uint4 v;
-        if (i < (uint32_t)SWEEP_CAP) v = g_sweep_smem[cand0 + i];
-        else v = __ldcg(spill + (i - SWEEP_CAP));
-        j = v.x; lo = v.y; cnt = v.z;
-    }
-    __device__ __forceinline__ void cand_sync() { __syncwarp(gmask); }
-    __device__ __forceinline__ void emit(uint32_t idx, MemEntry e) {
-        if (g == 0) __stcg(stage + idx, make_uint4(e.se, e.lo, e.cnt, e.sweep));
-    }
-    __device__ __forceinline__ void finish(uint32_t rid, uint32_t n) {
-        __syncwarp(gmask);
-        unsigned long long off = 0;
-        if (g == 0) off = atomicAdd(&a.counters[0], (unsigned long long)n);
-        off = __shfl_sync(gmask, off, gbase);
-        if (off + n > a.mem_cap) {
-            if (g == 0) { atomicOr(&a.counters[2], 1ull); a.mem_off[rid] = 0; a.mem_cnt[rid] = 0; }
-            return;
-        }
-        for (uint32_t k = g; k < n; k += SWEEP_LPR) a.mem_pool[off + k] = __ldcg(stage + k);
-        if (g == 0) { a.mem_off[rid] = (uint32_t)off; a.mem_cnt[rid] = n; }
-    }
-};
-
-// one byte per base, rounded up to 16 bytes
-__host__ __device__ inline uint32_t sweep_read_u4(uint32_t max_len) { return (max_len + 15u) / 16u; }
-
-__global__ void __launch_bounds__(SWEEP_THREADS, SWEEP_MIN_BLOCKS) k_sweep(const SweepArgs a) {
-    const uint32_t lane = threadIdx.x & 31u;
-    const uint32_t g = lane & 1u;
-    const uint32_t pair_in_block = threadIdx.x >> 1;
-    const uint32_t pair_u4 = SWEEP_CAP + a.read_u4 + a.pack_u4;
-    const uint32_t p0 = pair_in_block * pair_u4;
-    const size_t gp = (size_t)blockIdx.x * SWEEP_GROUPS + pair_in_block;
-    DevSweepCtx ctx{a, p0, (p0 + SWEEP_CAP) * 16u, (p0 + SWEEP_CAP + a.read_u4) * 4u, a.scratch + gp * 2 * a.max_len,
-                    a.scratch + gp * 2 * a.max_len + a.max_len, g, 3u << (lane & ~1u), lane & ~1u};
-    Sweeper<DevSweepCtx> sw;
-    for (;;) {
-        const bool need = sw.next(ctx, a.meta);
-        if (!__any_sync(0xFFFFFFFFu, need)) break;
-        // ONE uniform memory section per iteration: every pair issues its pending fetch here -- a seed-table entry
-        // or the (at most two) buckets of an FM step -- so all 16 chains' loads are in flight together.
-        const bool is_seed = need && sw.pending_seed();
-        const bool is_step = need && !is_seed;
-        uint4 se = make_uint4(0u, 0u, 0u, 0u);
-        if (is_seed) se = ldg_seed(a.seed_tab + sw.P0);
-        const bool rev = sw.on_reverse();
-        const StepOut r = pair_step(rev ? a.rev : a.fwd, sw.P0, sw.P0 + sw.cnt, sw.ch, a.meta.C[sw.ch & 3u],
-                                    rev ? a.meta.prim_r : a.meta.prim_f, g, is_step);
-        if (is_step) sw.consume(ctx, a.meta, r);
-        else if (is_seed) sw.consume_seed(ctx, a.meta, SeedEntry{se.x, se.y, se.z, se.w});
-    }
-}
-
 // ------------------------------------------------------------------------------------------------ one lane per read
-// The same sweep with ONE lane per read: every lane fetches whole 64-byte buckets itself (two 256-bit loads) and
-// popcounts all 192 symbols, so a warp-wide instruction of the uniform section advances 32 FM chains instead of 16, no
-// shuffles are needed, and the divergent per-read control is amortised over twice as many steps.  The kernel is bound
-// by instruction issue (profiles/r01_notes.md), which is what the quad -> pair change already showed; this is the next
-// halving.  Same Sweeper logic (sweep_logic.cuh), same outputs; chosen at run time (gsm_smem_sweep, GSM_SWEEP_LPR).
+// Every lane fetches whole 64-byte buckets itself (two 256-bit loads) and popcounts all 192 symbols, so a warp-wide
+// instruction of the uniform section advances 32 FM chains, no shuffles are needed, and the divergent per-read control is
+// amortised over 32 reads.  The kernel is bound by instruction issue (profiles/r01_notes.md).
 constexpr int SWEEP1_THREADS = 128;
 constexpr int SWEEP1_CAP = 8;                              // candidates kept in shared memory per read
 constexpr int SWEEP1_MIN_BLOCKS = 7;                       // register budget: 72 per thread (measured best of 6 / 7 / 8, profiles/r02_notes.md)
@@ -225,39 +109,18 @@ struct LanePartial {
     bool have;
 };
 
-// PAIRED: the two 32-byte halves of a lane's bucket are fetched by the lane and its neighbour with ONE load instruction
-// (lane g == r owns round r and loads half 0 of its bucket, the neighbour loads half 1 of the same bucket; eight shuffles
-// hand that half over), so a bucket is one 64-byte L2 request instead of two 32-byte ones.  The memory system sustains a
-// fixed RATE of random requests (about 58 G/s over a 667 MB index, tools/gather_ceiling.py) whatever their size up to 64
-// bytes.  PAIRED = false (the default: measured faster, profiles/r02_notes.md): the lane loads both halves itself.
-template <bool PAIRED>
+// The lane loads both halves of its bucket itself.  Fetching a bucket as one 64-byte request by a lane pair (shuffles hand
+// the other half over) measured slower: 54.7 vs 44.3 ms per 10 M reads at C4, the shuffles sit between the loads and their
+// use (profiles/r02_notes.md).
 __device__ __forceinline__ bool lane_step(const uint4* __restrict__ fwd, const uint4* __restrict__ rev, bool use_rev, uint32_t P0, uint32_t P1,
                                           uint32_t ch, uint32_t Cc, uint32_t primary, bool active, LanePartial& part, StepOut& out) {
-    constexpr uint32_t FULLM = 0xFFFFFFFFu;
     uint32_t b0, r0, b1, r1;
     split192(P0, b0, r0);
     split192(P1, b1, r1);
     const bool second = part.have;
     const uint32_t b = second ? b1 : b0;
     Half a0 = Half{0, 0, 0, 0, 0, 0, 0, 0}, a1 = a0;
-    if (PAIRED) {
-        const uint32_t g = threadIdx.x & 1u;
-        const uint32_t mine = (active ? 1u : 0u) | (use_rev ? 2u : 0u);
-        const uint32_t pb = __shfl_xor_sync(FULLM, b, 1);
-        const uint32_t theirs = __shfl_xor_sync(FULLM, mine, 1);
-#pragma unroll
-        for (uint32_t r = 0; r < 2u; ++r) {
-            const bool own = g == r;
-            const uint32_t bb = own ? b : pb, fl = own ? mine : theirs;
-            Half h = Half{0, 0, 0, 0, 0, 0, 0, 0};
-            if (fl & 1u) h = ldg_half((fl & 2u) ? rev : fwd, (size_t)bb * 2 + (own ? 0u : 1u));
-            Half o;
-            o.c0 = __shfl_xor_sync(FULLM, h.c0, 1); o.c1 = __shfl_xor_sync(FULLM, h.c1, 1);
-            o.l0 = __shfl_xor_sync(FULLM, h.l0, 1); o.l1 = __shfl_xor_sync(FULLM, h.l1, 1); o.l2 = __shfl_xor_sync(FULLM, h.l2, 1);
-            o.h0 = __shfl_xor_sync(FULLM, h.h0, 1); o.h1 = __shfl_xor_sync(FULLM, h.h1, 1); o.h2 = __shfl_xor_sync(FULLM, h.h2, 1);
-            if (own) { a0 = h; a1 = o; }
-        }
-    } else if (active) {
+    if (active) {
         const uint4* bk = use_rev ? rev : fwd;
         a0 = ldg_half(bk, (size_t)b * 2);
         a1 = ldg_half(bk, (size_t)b * 2 + 1);
@@ -286,10 +149,6 @@ __device__ __forceinline__ bool lane_step(const uint4* __restrict__ fwd, const u
     return true;
 }
 
-// LONG = false: the packed read is staged in shared memory (reads up to SWEEP1_SMEM_MAX_LEN bases).
-// LONG = true : the bases are read from the packed batch in global memory (L1 / L2 hits: 4 bases per byte), shared
-//               memory only holds the candidate slots, so any length up to 65535 runs; the grid is sized so that the
-//               per-lane match / candidate staging (2 x max_len x 16 bytes) fits a fixed budget.
 // flush_finished for a list of 33..64 matches (one read in a dozen at 1 % substitutions): same ordered, field-by-field
 // hand-over with two entries per lane -- entry x sits in lane x & 31 (x < 32: v0, else v1).  Out of line: its registers
 // are not the sweep loop's.
@@ -489,13 +348,13 @@ inline size_t sweep1_smem_bytes(uint32_t max_len, bool long_reads) {
     return (size_t)SWEEP1_THREADS * sweep1_lane_u4(max_len, long_reads) * sizeof(uint4) + 16;
 }
 
-// MB = resident blocks per SM the register allocation aims at (6: 80 registers, 7: 72, 8: 64 with spills); measured per
-// workload by tools/sweep_ab.py (GSM_SWEEP_BLOCKS)
-// STATS: count lane-slots / FM passes / seed fetches / text operations into counters[4..7] (measurement builds only)
-// PAIRED: buckets fetched as one 64-byte request by lane pairs (lane_step); measured slower than two requests per lane
-// (54.7 vs 44.3 ms per 10 M reads at C4: the shuffles sit between the loads and their use), kept as GSM_SWEEP_PAIRED=1
-template <bool LONG, bool UNIQ, int MB = SWEEP1_MIN_BLOCKS, bool STATS = false, bool PAIRED = false>
-__global__ void __launch_bounds__(SWEEP1_THREADS, MB) k_sweep1(const SweepArgs a) {
+// LONG = false: the packed read is staged in shared memory (reads up to SWEEP1_SMEM_MAX_LEN bases).
+// LONG = true : the bases are read from the packed batch in global memory (L1 / L2 hits: 4 bases per byte), shared
+//               memory only holds the candidate slots, so any length up to 65535 runs; the grid is sized so that the
+//               per-lane match / candidate staging (2 x max_len x 16 bytes) fits a fixed budget.
+// UNIQ  : the unique-match shortcut, for an index with the suffix array and the packed text on the device.
+template <bool LONG, bool UNIQ>
+__global__ void __launch_bounds__(SWEEP1_THREADS, SWEEP1_MIN_BLOCKS) k_sweep1(const SweepArgs a) {
     using Ctx = DevSweepCtx1<LONG, UNIQ>;
     const uint32_t lane_u4 = sweep1_lane_u4(a.max_len, LONG);
     const uint32_t p0 = threadIdx.x * lane_u4;
@@ -503,7 +362,6 @@ __global__ void __launch_bounds__(SWEEP1_THREADS, MB) k_sweep1(const SweepArgs a
     Ctx ctx{a, p0, (p0 + SWEEP1_CAP) * 4u, a.scratch + gl * 2 * a.max_len, a.scratch + gl * 2 * a.max_len + a.max_len, nullptr, 0u, Ctx::NO_FIN};
     Sweeper<Ctx> sw;
     LanePartial part{0u, 0u, false};
-    uint32_t n_it = 0, n_step = 0, n_seed = 0, n_text = 0;
     for (;;) {
         ctx.flush_finished();                 // reads finished by the last iteration's consume: before their lanes reuse the staging slots
         const bool need = sw.next(ctx, a.meta);
@@ -516,7 +374,6 @@ __global__ void __launch_bounds__(SWEEP1_THREADS, MB) k_sweep1(const SweepArgs a
         const bool is_word = UNIQ && need && sw.pending_word();
         const bool is_cmp = UNIQ && need && sw.pending_cmp();
         const bool is_step = need && !is_seed && !is_word && !is_cmp;
-        if (STATS) { n_it++; n_step += is_step; n_seed += is_seed; n_text += is_word || is_cmp; }
         uint4 se = make_uint4(0u, 0u, 0u, 0u);
         if (is_seed) se = ldg_seed(a.seed_tab + sw.P0);
         uint32_t wv = 0u, matched = 0u;
@@ -528,26 +385,13 @@ __global__ void __launch_bounds__(SWEEP1_THREADS, MB) k_sweep1(const SweepArgs a
         }
         const bool rev = sw.on_reverse();
         StepOut r;
-        const bool stepped = lane_step<PAIRED>(a.fwd, a.rev, rev, sw.P0, sw.P0 + sw.cnt, sw.ch, a.meta.C[sw.ch & 3u],
-                                               rev ? a.meta.prim_r : a.meta.prim_f, is_step, part, r);
+        const bool stepped = lane_step(a.fwd, a.rev, rev, sw.P0, sw.P0 + sw.cnt, sw.ch, a.meta.C[sw.ch & 3u],
+                                       rev ? a.meta.prim_r : a.meta.prim_f, is_step, part, r);
         if (stepped) sw.consume(ctx, a.meta, r);
         else if (is_seed) sw.consume_seed(ctx, a.meta, SeedEntry{se.x, se.y, se.z, se.w});
         else if (UNIQ && is_word) sw.consume_word(ctx, a.meta, wv);
         else if (UNIQ && is_cmp) sw.consume_cmp(ctx, a.meta, matched);
     }
-    if (STATS) {
-        atomicAdd(&a.counters[4], (unsigned long long)n_it);
-        atomicAdd(&a.counters[5], (unsigned long long)n_step);
-        atomicAdd(&a.counters[6], (unsigned long long)n_seed);
-        atomicAdd(&a.counters[7], (unsigned long long)n_text);
-    }
-}
-
-// packed words of a read, rounded up to 16-byte chunks
-__host__ __device__ inline uint32_t sweep_pack_u4(uint32_t max_len) { return (max_len + 63u) / 64u; }
-
-inline size_t sweep_smem_bytes(uint32_t max_len) {
-    return (size_t)SWEEP_GROUPS * (SWEEP_CAP + sweep_read_u4(max_len) + sweep_pack_u4(max_len)) * sizeof(uint4) + 16;
 }
 
 }  // namespace gsm

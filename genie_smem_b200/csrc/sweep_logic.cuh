@@ -74,14 +74,14 @@ constexpr uint32_t SWEEP_CMP_CHUNK = 64;   // bases compared per text fetch
 //   uint32_t seed_k()                                   K of the seed table, 0 = no table
 //   bool     uniq()                                     unique-match shortcut available: once q[x:pos) occurs exactly once
 //                                                       the forward extension follows the TEXT (one suffix-array fetch, then
-//                                                       64 bases per compare) instead of one FM step per base.  The lane
-//                                                       kernels (k_sweep1) run it; the pair kernel compiles it out.
+//                                                       64 bases per compare) instead of one FM step per base.  k_sweep1
+//                                                       runs it when the suffix array and the text are on the device.
 //   bool     uniq_back()                                also walk unique matches to the LEFT along the text (needs the inverse
 //                                                       suffix array; host-compiled test only)
 //   uint32_t kmer(uint32_t pos)                         code of q[pos:pos+K) (LUT.convert_seq_to_num, LUT.py:37-48)
 //   void     cand_put(uint32_t i, uint32_t j, uint32_t lo, uint32_t cnt)
 //   void     cand_get(uint32_t i, uint32_t& j, uint32_t& lo, uint32_t& cnt)
-//   void     cand_sync()                                make candidate writes visible to the pair
+//   void     cand_sync()                                make candidate writes visible to the read's other lanes, if any
 //   void     emit(uint32_t idx, MemEntry e)             stage maximal match #idx of this read
 //   void     finish(uint32_t rid, uint32_t n_mems)      read complete
 // BWA-SMEM selection (get_SMEMS, SMEM.py:456-467 = Selector::run_bwa) as a MAXIMUM over the ordered match list: standing at

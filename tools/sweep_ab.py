@@ -1,9 +1,8 @@
 #!/usr/bin/env python3
-"""A/B harness for kernel variants: the bench's index and reads at a reduced read count, per-kernel times (CUDA events)
-and a checksum of every method's records, as one JSON line.  Variants are chosen by environment (e.g. GSM_SWEEP_LPR),
-which the library reads once per process: run once per setting and compare the lines.
+"""A/B harness: the bench's index and reads at a reduced read count, per-kernel times (CUDA events) and a checksum of
+every method's records, as one JSON line.  Run it once per build and compare the lines.
 
-Usage: [GSM_SWEEP_LPR=1] python tools/sweep_ab.py [--reads N] [--ref-bases B] [--steps K] [--skip-rmi] [--tag name]"""
+Usage: python tools/sweep_ab.py [--reads N] [--ref-bases B] [--steps K] [--skip-rmi] [--tag name]"""
 import argparse
 import hashlib
 import json
@@ -63,13 +62,9 @@ def main():
         torch.cuda.synchronize()
         return e0.elapsed_time(e1) / steps
 
-    out = {"tag": a.tag, "env": {k: v for k, v in os.environ.items() if k.startswith("GSM_")}, "reads": a.reads, "ref_bases": a.ref_bases,
+    out = {"tag": a.tag, "reads": a.reads, "ref_bases": a.ref_bases,
            "seed_K": int(index.seed_K), "setup_s": round(setup, 1)}
     out["ms_sweep"] = round(timed(lambda: eng.sweep(batch), a.steps), 3)
-    if os.environ.get("GSM_SWEEP_STATS"):
-        c = eng.counters.cpu().numpy()
-        out["stats_per_read"] = {"lane_slots": round(float(c[4]) / a.reads, 2), "fm_passes": round(float(c[5]) / a.reads, 2),
-                                 "seed_fetches": round(float(c[6]) / a.reads, 2), "text_ops": round(float(c[7]) / a.reads, 2)}
     legs = [("bwa", g.METHOD_BWA, {"min_len": 1}), ("lut", g.METHOD_LUT, {"K": bench.LUT_K, "lut": lut}),
             ("lut_machine", g.METHOD_LUT, {"K": bench.LUT_K, "lut": lut})]
     if rmi is not None:
